@@ -2,7 +2,7 @@
 """Benchmark of the north-star metric: windows/sec, M-best, N=4096, Pmax=1024, num=10 (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--windows B_PER_GPU]
-                    [--secondary all|none|2,3g,4,5qo,5ram]
+                    [--secondary all|none|2,3g,4,5qo,5ram] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A *step* is one pass of Periods.m_best(num=10, max_length=1024) over one batch of synthetic
@@ -137,6 +137,31 @@ class OraclePool:
 
 def sample_windows(stream: np.ndarray, count: int):
     return [np.array(stream[HOP * b: HOP * b + N_WIN]) for b in range(count)]
+
+
+# under 64 MB in all with the .npy headers
+DUMP_BYTES = 60_000_000
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Write each per-window result array (first axis = window) as out_dir/<name>.npy in float64, which holds the int32
+    periods and counts exactly.  When the arrays would exceed DUMP_BYTES together, every array keeps the same fixed,
+    seeded sample of windows, and their indices are written as rows.npy."""
+    import torch
+    arrays = {k: v.view(torch.int32) if v.dtype == getattr(torch, "uint32", None) else v for k, v in arrays.items()}
+    b = next(iter(arrays.values())).shape[0]
+    row_bytes = 8 * sum(v[0].numel() for v in arrays.values())
+    rows = None
+    if b * row_bytes > DUMP_BYTES:
+        keep = DUMP_BYTES // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(0).choice(b, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        if rows is not None:
+            v = v[torch.from_numpy(rows).to(v.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), v.cpu().numpy().astype(np.float64))
+    if rows is not None:
+        np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -679,6 +704,9 @@ def run_b200(args, rank: int, world: int, local_rank: int):
     sweeps = int(res.sweeps.sum().item())
     status_bad = int((res.status != 0).sum().item())
     near_tie_windows = int((res.near_ties != 0).sum().item())
+    if args.dump_outputs and rank == 0:   # the last timed step's results (rank 0's windows when several GPUs run)
+        dump_outputs(args.dump_outputs, {"periods": res.periods, "powers": res.powers, "status": res.status,
+                                         "sweeps": res.sweeps, "near_ties": res.near_ties})
 
     # ---- end-to-end through the public API with pinned host buffers: every step timed on its own, median reported
     e2e_steps = max(1, args.e2e_steps)
@@ -853,7 +881,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--secondary", default="all",
                     help="other BASELINE configs appended to the line: all | none | comma list of 2,3g,4,5qo,5ram")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the M-best results of the last timed step as DIR/<name>.npy (float64; a fixed sample of "
+                         "windows above 60 MB); the same arguments give the same inputs, so two builds compare output "
+                         "for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
