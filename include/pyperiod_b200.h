@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PP_ABI_VERSION 5
+#define PP_ABI_VERSION 6
 
 /* sweep metrics */
 #define PP_METRIC_NORM 0   /* ||proj_p|| / sqrt(N)                 Periods.py:221-241, 507-508 */
@@ -56,6 +56,8 @@ extern "C" {
 #define PP_ALGO_BCORR 3
 #define PP_ALGO_QO 4
 #define PP_ALGO_RAMANUJAN 5
+#define PP_ALGO_PROJECT 6
+#define PP_ALGO_BFREQ 7
 
 int pp_abi_version(void);
 const char *pp_last_error(void);
@@ -173,6 +175,51 @@ int pp_best_frequency_round(double *work, int32_t B, int32_t N, const double *ma
                             int32_t trunc, int32_t orth, const int32_t *chain_off, const int32_t *chain_q,
                             int32_t table_pmax, uint32_t *periods, double *norms, double *bases, int32_t round,
                             int32_t num, int32_t *status, void *stream);
+
+/* ---- the global-memory ("long") path of the Periods family -------------------------------------------------
+ * The on-chip entry points above stage the whole window, the single-period vectors and the sweep scratch of one
+ * window in one CTA's shared memory and return -2 when that plan does not fit.  pp_fits_on_chip answers, without
+ * touching a device, whether the on-chip plan of a call fits `smem_bytes` (the device's opt-in shared memory per
+ * block): 1 = fits, 0 = does not, < 0 = bad arguments.  algo: PP_ALGO_PROJECT (pmax = p), PP_ALGO_SWEEP,
+ * PP_ALGO_MBEST (metric NORM or GAMMA), PP_ALGO_S2L (pmax = n_periods), PP_ALGO_BCORR (pmax = max_length) or
+ * PP_ALGO_BFREQ (pmax unused); metric / trunc / orth / fold_mode are the call's own (they decide which sweep
+ * scratch the plan holds).
+ *
+ * pp_long_* take the arguments of the on-chip entry point of the same name and return the same results for any
+ * window length: residuals are copied to the workspace (the input is never written), every sweep is spread over the
+ * whole GPU as one work unit per (window, candidate period), and each window's selection step runs in one CTA.  The
+ * host drives the rounds on `stream` and reads a 4-byte active-window count once per round, so these calls return
+ * after their work is done except pp_long_project and pp_long_best_frequency_round, which only enqueue.  Ranking
+ * sweeps fold directly (sequential fp64 sums, the fold_mode of the on-chip call has no counterpart), so M-best in
+ * every fold mode and dtype selects the periods and powers of the fp64 direct fold.  Workspace:
+ * pp_long_workspace_bytes(algo, B, N, pmax, num, orth), with pmax as for pp_fits_on_chip (N for PP_ALGO_BFREQ). */
+int pp_fits_on_chip(int32_t algo, int32_t N, int32_t pmax, int32_t num, int32_t metric, int32_t trunc, int32_t orth,
+                    int32_t fold_mode, int32_t smem_bytes);
+size_t pp_long_workspace_bytes(int32_t algo, int32_t B, int32_t N, int32_t pmax, int32_t num, int32_t orth);
+int pp_long_project(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t p, int32_t trunc,
+                    const int32_t *chain_q_host, int32_t chain_len, double *out, int64_t ldo, int32_t out_len,
+                    void *workspace, size_t workspace_bytes, void *stream);
+int pp_long_sweep(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t pmin, int32_t pmax, int32_t metric,
+                  int32_t trunc, int32_t orth, const int32_t *chain_off, const int32_t *chain_q, int32_t table_pmax,
+                  double *metric_out, int32_t *best_p, double *best_val, void *workspace, size_t workspace_bytes,
+                  void *stream);
+int pp_long_mbest(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t num, int32_t pmin, int32_t pmax,
+                  int32_t gamma, int32_t trunc, int32_t orth, const int32_t *chain_off, const int32_t *chain_q,
+                  const int32_t *fac_off, const int32_t *fac, int32_t table_pmax, uint32_t *periods, double *powers,
+                  double *bases, int32_t *sweeps, int32_t *near_ties, int32_t *status, void *workspace,
+                  size_t workspace_bytes, void *stream);
+int pp_long_small_to_large(const double *x, int64_t ldx, int32_t B, int32_t N, double thresh, int32_t n_periods,
+                           int32_t trunc, int32_t orth, const int32_t *chain_off, const int32_t *chain_q,
+                           int32_t table_pmax, int32_t kmax, uint32_t *periods, double *powers, double *bases,
+                           int32_t *count, int32_t *status, void *workspace, size_t workspace_bytes, void *stream);
+int pp_long_best_correlation(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t num, int32_t max_length,
+                             double ratio, int32_t trunc, int32_t orth, const int32_t *chain_off,
+                             const int32_t *chain_q, int32_t table_pmax, uint32_t *periods, double *powers,
+                             double *bases, int32_t *status, void *workspace, size_t workspace_bytes, void *stream);
+int pp_long_best_frequency_round(double *work, int32_t B, int32_t N, const double *mags, int32_t F, int32_t win_size,
+                                 int32_t trunc, int32_t orth, const int32_t *chain_off, const int32_t *chain_q,
+                                 int32_t table_pmax, uint32_t *periods, double *norms, double *bases, int32_t round,
+                                 int32_t num, int32_t *status, void *workspace, size_t workspace_bytes, void *stream);
 
 /* ---- QOPeriods.find_periods, default branch (QOPeriods.py:313-643, 743-852) ---------------
  * Per window up to `num` rounds: gamma-norm sweep of the residual over [pmin, pmax]

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PYPERIOD_B200_LIB selects an alternative build of the same library (kernel tuning experiments)
 LIB_PATH = os.environ.get("PYPERIOD_B200_LIB") or os.path.join(HERE, "libpyperiod_b200.so")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 METRIC_NORM, METRIC_GAMMA, METRIC_MAXABS, METRIC_IMPOSED = 0, 1, 2, 3
 STATUS_OK, STATUS_NO_PERIOD, STATUS_OVERFLOW, STATUS_SINGULAR, STATUS_GUARD = 0, 1, 2, 3, 4
@@ -20,6 +20,7 @@ STATUS_TOO_LARGE, STATUS_ZERO_INPUT = 5, 6
 BASIS_NATURAL, BASIS_RAMANUJAN = 0, 1
 RAM_FP64, RAM_TF32, RAM_F32COMPAT = 0, 1, 2
 ALGO_SWEEP, ALGO_MBEST, ALGO_S2L, ALGO_BCORR, ALGO_QO, ALGO_RAMANUJAN = 0, 1, 2, 3, 4, 5
+ALGO_PROJECT, ALGO_BFREQ = 6, 7
 
 _p = C.c_void_p
 _i32 = C.c_int32
@@ -69,6 +70,19 @@ SIGNATURES = {
                               _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
     "pp_qo_get_periods": (C.c_int, [_i32, _i32, _i32, _i32, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _p, _p]),
     "pp_qo_dictionary_rows": (C.c_int, [_i32, _i32, _p, _p, _i32, _p, _i32, _p, _p]),
+    "pp_fits_on_chip": (C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32]),
+    "pp_long_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i32, _i32]),
+    "pp_long_project": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _p, _i32, _p, _i64, _i32, _p, _sz, _p]),
+    "pp_long_sweep": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _i32, _p, _p, _p, _p, _sz,
+                                _p]),
+    "pp_long_mbest": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _i32,
+                                _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "pp_long_small_to_large": (C.c_int, [_p, _i64, _i32, _i32, _f64, _i32, _i32, _i32, _p, _p, _i32, _i32,
+                                         _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "pp_long_best_correlation": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _f64, _i32, _i32, _p, _p, _i32,
+                                           _p, _p, _p, _p, _p, _sz, _p]),
+    "pp_long_best_frequency_round": (C.c_int, [_p, _i32, _i32, _p, _i32, _i32, _i32, _i32, _p, _p, _i32, _p, _p, _p,
+                                               _i32, _i32, _p, _p, _sz, _p]),
     "pp_qo_solve_rows": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _p, _i32, _i32, _i32, _p, _p, _i64, _p, _p, _p,
                                    _sz, _p]),
 }
@@ -161,6 +175,17 @@ def microbench(kind: int, iters: int = 4000) -> dict:
     out = (C.c_double * 3)()
     check(load().pp_microbench(kind, iters, out), "pp_microbench")
     return {"per_s": out[0], "sm_mhz": out[1], "ms": out[2]}
+
+
+def fits_on_chip(algo: int, n: int, pmax: int, num: int, metric: int, trunc: int, orth: int, fold_mode: int,
+                 smem_bytes: int) -> bool:
+    """Whether the on-chip plan of a call fits `smem_bytes` of shared memory per block (pp_fits_on_chip; no device
+    is touched).  Calls whose plan does not fit run on the global-memory path (pp_long_*)."""
+    rc = load().pp_fits_on_chip(int(algo), int(n), int(pmax), int(num), int(metric), int(trunc), int(orth),
+                                int(fold_mode), int(smem_bytes))
+    if rc < 0:
+        check(rc, "pp_fits_on_chip")
+    return rc == 1
 
 
 def device_info() -> dict:

@@ -25,6 +25,12 @@ struct BfPlan {
   __host__ __device__ size_t bytes() const { return off_bar() + 32; }
 };
 
+size_t bfreq_smem_bytes(int N) {
+  BfPlan pl;
+  pl.n_even = (N + 1) & ~1;
+  return pl.bytes();
+}
+
 __global__ void __launch_bounds__(kThreads, 2)
 bfreq_round_kernel(double* __restrict__ work, int B, int N, const double* __restrict__ mags, int F, int win, int trunc,
                    int orth, const int32_t* __restrict__ chain_off, const int32_t* __restrict__ chain_q, int table_pmax,

@@ -12,6 +12,9 @@ namespace pp {
 int fail(int code, const char* fmt, const char* a = "");
 int check_cuda(cudaError_t e, const char* what);
 
+// shared memory of bfreq_round_kernel for windows of N samples (pp_bfreq.cu)
+size_t bfreq_smem_bytes(int N);
+
 // fold modes are per-call arguments (include/pyperiod_b200.h)
 static inline int check_fold_mode(int mode) {
   if (mode < 0 || mode > 3) return fail(-1, "unknown fold mode%s");

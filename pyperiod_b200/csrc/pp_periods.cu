@@ -926,6 +926,32 @@ size_t pp_workspace_bytes(int32_t algo, int32_t N, int32_t pmax, int32_t num, in
   return bytes;
 }
 
+int pp_fits_on_chip(int32_t algo, int32_t N, int32_t pmax, int32_t num, int32_t metric, int32_t trunc, int32_t orth,
+                    int32_t fold_mode, int32_t smem_bytes) {
+  if (N < 1 || pmax < 0 || num < 0 || metric < 0 || metric > 3 || smem_bytes < 0) return fail(-1, "bad arguments%s");
+  if (check_fold_mode(fold_mode)) return -1;
+  size_t bytes = 0;
+  switch (algo) {
+    case PP_ALGO_PROJECT: bytes = make_plan(N, pmax, 0, false).bytes(); break;
+    case PP_ALGO_SWEEP:
+      bytes = make_plan(N, pmax, 0, true, hier_applies(fold_mode, metric, trunc, orth), false,
+                        metric == PP_METRIC_NORM || metric == PP_METRIC_GAMMA).bytes();
+      break;
+    case PP_ALGO_MBEST: {
+      const bool hier = hier_applies(fold_mode, metric, trunc, orth);
+      bytes = make_plan(N, pmax, num, true, hier, hier && !trunc && fold_mode == PP_FOLD_NOMINATE_F32, true).bytes();
+      break;
+    }
+    case PP_ALGO_S2L: bytes = make_plan(N, pmax, 0, true).bytes(); break;
+    case PP_ALGO_BCORR:
+      bytes = make_plan(N, pmax, 0, true, fold_mode != PP_FOLD_DIRECT && pmax - 1 >= 4).bytes();
+      break;
+    case PP_ALGO_BFREQ: bytes = bfreq_smem_bytes(N); break;
+    default: return fail(-1, "unknown algorithm%s");
+  }
+  return bytes <= (size_t)smem_bytes ? 1 : 0;
+}
+
 static int check_common(const void* x, int64_t ldx, int B, int N) {
   if (x == nullptr) return fail(-1, "x is null%s");
   if (B < 0 || N < 2) return fail(-1, "need B >= 0 and N >= 2%s");

@@ -61,6 +61,31 @@ def _is_data(obj) -> bool:
     return isinstance(obj, (np.ndarray, list, tuple)) and np.ndim(obj) >= 1
 
 
+STAGINGS = ("auto", "shared", "global")
+_smem_optin: dict = {}
+
+
+def _check_staging(staging):
+    if staging not in STAGINGS:
+        raise ValueError("staging must be 'auto', 'shared' or 'global'")
+
+
+def _global_staging(staging, device, algo, n, pmax, num=0, metric=0, trunc=False, orth=False,
+                    fold=_lib.FOLD_DIRECT) -> bool:
+    """Whether a call runs on the global-memory path: forced by staging="global", never with "shared", and with
+    "auto" exactly when the on-chip plan of the call does not fit the device's opt-in shared memory per block."""
+    if staging == "global":
+        return True
+    if staging == "shared":
+        return False
+    key = str(device)
+    if key not in _smem_optin:
+        with torch.cuda.device(device):
+            _smem_optin[key] = _lib.device_info()["smem_optin_bytes"]
+    return not _lib.fits_on_chip(algo, n, pmax, num, metric, int(bool(trunc)), int(bool(orth)), fold,
+                                 _smem_optin[key])
+
+
 def _u32(t: torch.Tensor):
     return t.view(torch.uint32) if hasattr(torch, "uint32") else t
 
@@ -78,14 +103,21 @@ class Periods:
     """Sethares-Staley periodicity transforms, B200-native.  See module docstring."""
 
     def __init__(self, *args, trunc_to_integer_multiple=None, orthogonalize=None, device=None, dtype="fp64",
-                 fold_mode=None, devices=None):
+                 fold_mode=None, devices=None, staging="auto"):
         """device / devices / dtype / fold_mode are not part of the reference API.  devices=[...] (CUDA device indices
         or names) shards a host (B, N) batch over several GPUs from ONE process: contiguous blocks of windows, one
         worker thread and one set of launches per device, results concatenated on the host (windows are independent:
         no collective; the one-process-per-GPU form of the same sharding is pyperiod_b200.sharding).  dtype="fp32" ranks the M-best sweeps in float
         (half the shared-memory traffic) and re-folds every candidate inside the float error bound in fp64, so the
         period lists and norms are those of the fp64 path (the north star's fp32 option).  fold_mode (a
-        _lib.FOLD_* value or name) picks how ranking sweeps obtain the residue sums; None = the module default."""
+        _lib.FOLD_* value or name) picks how ranking sweeps obtain the residue sums; None = the module default.
+
+        staging picks where a window lives while it is processed.  "shared" stages it in one CTA's shared memory (the
+        on-chip kernels; a window whose plan does not fit raises PPError).  "global" runs the global-memory path: the
+        residual stays in a device workspace and every sweep is spread over the whole GPU, for windows of any length.
+        "auto" (default) takes the on-chip path whenever its plan fits the device and the global path otherwise.  The
+        global path ranks with direct fp64 folds: in every fold_mode and with dtype="fp32" it selects the periods and
+        powers of the fp64 path (powers can differ from the hierarchical on-chip sweep in the last bits)."""
         args = list(args)
         self._data = None
         if args and _is_data(args[0]):
@@ -109,6 +141,8 @@ class Periods:
             raise ValueError("dtype must be 'fp64' or 'fp32'")
         self._dtype = dtype
         self._fold_mode = fold_mode
+        _check_staging(staging)
+        self._staging = staging
         _lib.load()  # fail loudly now if the CUDA library is missing
 
     def _fold(self) -> int:
@@ -137,7 +171,7 @@ class Periods:
         def work(i):
             lo, hi = shard_bounds(b, len(devs), i)
             sub = Periods(self._trunc_to_integer_multiple, self._orthogonalize, device=devs[i], dtype=self._dtype,
-                          fold_mode=self._fold_mode)
+                          fold_mode=self._fold_mode, staging=self._staging)
             return getattr(sub, name)(data[lo:hi], *rest, **kw)   # row slices keep hop-framed (overlapping) strides
 
         with ThreadPoolExecutor(len(devs)) as pool:
@@ -176,11 +210,12 @@ class Periods:
     # ------------------------------------------------------------------ static operators
     @staticmethod
     def project(data, p=2, trunc_to_integer_multiple=False, orthogonalize=False, return_single_period=False,
-                device=None):
+                device=None, staging="auto"):
         """Projection onto the p-periodic subspace (Periods.py:142-219); bit-exact with the reference.
 
-        1-D -> (N,) (or (p,) with return_single_period); (B, N) -> (B, N) / (B, p).
+        1-D -> (N,) (or (p,) with return_single_period); (B, N) -> (B, N) / (B, p).  staging: see Periods().
         """
+        _check_staging(staging)
         lib = _lib.load()
         w = stage_windows(data, device)
         p = int(p)
@@ -200,9 +235,15 @@ class Periods:
             return res[0] if w.was_1d else res
         chain = np.asarray(orth_chain(p) if orthogonalize else [], dtype=np.int32)
         out = torch.empty((w.b, out_len), dtype=torch.float64, device=w.device)
-        call(lib.pp_project, "pp_project", w.device, ptr(w.tensor), w.ldx, w.b, w.n, p,
-             int(bool(trunc_to_integer_multiple)), chain.ctypes.data_as(C.c_void_p), len(chain), ptr(out), out_len,
-             out_len, stream_ptr(w.device))
+        if _global_staging(staging, w.device, _lib.ALGO_PROJECT, w.n, p):
+            ws = workspace_for(w.device, lib.pp_long_workspace_bytes, _lib.ALGO_PROJECT, w.b, w.n, p, 0, 0)
+            call(lib.pp_long_project, "pp_long_project", w.device, ptr(w.tensor), w.ldx, w.b, w.n, p,
+                 int(bool(trunc_to_integer_multiple)), chain.ctypes.data_as(C.c_void_p), len(chain), ptr(out), out_len,
+                 out_len, ptr(ws), ws.numel(), stream_ptr(w.device))
+        else:
+            call(lib.pp_project, "pp_project", w.device, ptr(w.tensor), w.ldx, w.b, w.n, p,
+                 int(bool(trunc_to_integer_multiple)), chain.ctypes.data_as(C.c_void_p), len(chain), ptr(out), out_len,
+                 out_len, stream_ptr(w.device))
         res = _export(w, out)
         return res[0] if w.was_1d else res
 
@@ -236,10 +277,16 @@ class Periods:
         orth = self._orthogonalize and metric != 2
         tb = get_tables(pmax)
         co, cq, _, _ = tb.device(w.device)
-        ws = workspace_for(w.device, lib.pp_workspace_bytes, _lib.ALGO_SWEEP, w.n, pmax, 0, int(orth))
         metrics = torch.zeros((w.b, pmax + 1), dtype=torch.float64, device=w.device)
         best_p = torch.empty((w.b,), dtype=torch.int32, device=w.device)
         best_v = torch.empty((w.b,), dtype=torch.float64, device=w.device)
+        if _global_staging(self._staging, w.device, _lib.ALGO_SWEEP, w.n, pmax, 0, metric, trunc, orth, self._fold()):
+            ws = workspace_for(w.device, lib.pp_long_workspace_bytes, _lib.ALGO_SWEEP, w.b, w.n, pmax, 0, int(orth))
+            call(lib.pp_long_sweep, "pp_long_sweep", w.device, ptr(w.tensor), w.ldx, w.b, w.n, pmin, pmax, metric,
+                 int(trunc), int(orth), ptr(co), ptr(cq), tb.pmax, ptr(metrics), ptr(best_p), ptr(best_v), ptr(ws),
+                 ws.numel(), stream_ptr(w.device))
+            return _export(w, metrics), _export(w, best_p), _export(w, best_v)
+        ws = workspace_for(w.device, lib.pp_workspace_bytes, _lib.ALGO_SWEEP, w.n, pmax, 0, int(orth))
         call(lib.pp_sweep, "pp_sweep", w.device, ptr(w.tensor), w.ldx, w.b, w.n, pmin, pmax, metric, int(trunc),
              int(orth), self._fold(), ptr(co), ptr(cq), tb.pmax, ptr(metrics), ptr(best_p), ptr(best_v), ptr(ws),
              ws.numel(), stream_ptr(w.device))
@@ -278,7 +325,14 @@ class Periods:
         tb = get_tables(pmax)
         co, cq, fo, fc = tb.device(w.device)
         orth = int(self._orthogonalize)
-        ws = workspace_for(w.device, lib.pp_workspace_bytes, _lib.ALGO_MBEST, w.n, pmax, num, orth)
+        fold = self._fold()
+        trunc = int(self._trunc_to_integer_multiple)
+        metric = _lib.METRIC_GAMMA if gamma else _lib.METRIC_NORM
+        long = _global_staging(self._staging, w.device, _lib.ALGO_MBEST, w.n, pmax, num, metric, trunc, orth, fold)
+        if long:
+            ws = workspace_for(w.device, lib.pp_long_workspace_bytes, _lib.ALGO_MBEST, w.b, w.n, pmax, num, orth)
+        else:
+            ws = workspace_for(w.device, lib.pp_workspace_bytes, _lib.ALGO_MBEST, w.n, pmax, num, orth)
         periods = torch.empty((w.b, num), dtype=torch.int32, device=w.device)
         powers = torch.empty((w.b, num), dtype=torch.float64, device=w.device)
         bases = torch.empty((w.b, num, w.n), dtype=torch.float64, device=w.device) if return_bases else None
@@ -286,10 +340,16 @@ class Periods:
         near = torch.empty((w.b,), dtype=torch.int32, device=w.device)
         status = torch.empty((w.b,), dtype=torch.int32, device=w.device)
         cur = torch.cuda.current_stream(w.device)
-        fold = self._fold()
         for b0, b1, ready in w.launch_plan():
             if ready is not None:
                 cur.wait_event(ready)
+            if long:
+                call(lib.pp_long_mbest, "pp_long_mbest", w.device, C.c_void_p(w.ptr + b0 * w.ldx * 8), w.ldx, b1 - b0,
+                     w.n, num, min_length, pmax, int(gamma), trunc, orth, ptr(co), ptr(cq), ptr(fo), ptr(fc), tb.pmax,
+                     ptr(periods[b0:b1]), ptr(powers[b0:b1]), ptr(None if bases is None else bases[b0:b1]),
+                     ptr(sweeps[b0:b1]), ptr(near[b0:b1]), ptr(status[b0:b1]), ptr(ws), ws.numel(),
+                     stream_ptr(w.device))
+                continue
             call(lib.pp_mbest, "pp_mbest", w.device, C.c_void_p(w.ptr + b0 * w.ldx * 8), w.ldx, b1 - b0, w.n, num,
                  min_length, pmax, int(gamma), int(self._trunc_to_integer_multiple), orth, fold, ptr(co), ptr(cq),
                  ptr(fo), ptr(fc), tb.pmax, ptr(periods[b0:b1]), ptr(powers[b0:b1]),
@@ -329,7 +389,15 @@ class Periods:
         tb = get_tables(n_periods)
         co, cq, _, _ = tb.device(w.device)
         orth = int(self._orthogonalize)
-        ws = workspace_for(w.device, lib.pp_workspace_bytes, _lib.ALGO_S2L, w.n, n_periods, 0, orth)
+        trunc = int(self._trunc_to_integer_multiple)
+        long = _global_staging(self._staging, w.device, _lib.ALGO_S2L, w.n, n_periods, 0, _lib.METRIC_IMPOSED, trunc,
+                               orth)
+        if long:
+            ws = workspace_for(w.device, lib.pp_long_workspace_bytes, _lib.ALGO_S2L, w.b, w.n, n_periods, 0, orth)
+        else:
+            ws = workspace_for(w.device, lib.pp_workspace_bytes, _lib.ALGO_S2L, w.n, n_periods, 0, orth)
+        fn, name = (lib.pp_long_small_to_large, "pp_long_small_to_large") if long else \
+            (lib.pp_small_to_large, "pp_small_to_large")
         cur = torch.cuda.current_stream(w.device)
         plan = list(w.launch_plan()) if w.plan is None else None   # a pipelined plan issues its copies as it is walked
         while True:
@@ -341,8 +409,8 @@ class Periods:
             for b0, b1, ready in (plan if plan is not None else w.launch_plan()):
                 if ready is not None:
                     cur.wait_event(ready)
-                call(lib.pp_small_to_large, "pp_small_to_large", w.device, C.c_void_p(w.ptr + b0 * w.ldx * 8), w.ldx,
-                     b1 - b0, w.n, thresh, n_periods, int(self._trunc_to_integer_multiple), orth, ptr(co), ptr(cq),
+                call(fn, name, w.device, C.c_void_p(w.ptr + b0 * w.ldx * 8), w.ldx,
+                     b1 - b0, w.n, thresh, n_periods, trunc, orth, ptr(co), ptr(cq),
                      tb.pmax, kmax, ptr(periods[b0:b1]), ptr(powers[b0:b1]), ptr(None if bases is None else bases[b0:b1]),
                      ptr(count[b0:b1]), ptr(status[b0:b1]), ptr(ws), ws.numel(), stream_ptr(w.device))
             if not w.was_1d:
@@ -380,12 +448,24 @@ class Periods:
         powers = torch.empty((w.b, num), dtype=torch.float64, device=w.device)
         bases = torch.empty((w.b, num, w.n), dtype=torch.float64, device=w.device) if return_bases else None
         status = torch.empty((w.b,), dtype=torch.int32, device=w.device)
-        ws = workspace_for(w.device, lib.pp_workspace_bytes, _lib.ALGO_BCORR, w.n, max_length, num,
-                           int(self._orthogonalize))
+        trunc, orth = int(self._trunc_to_integer_multiple), int(self._orthogonalize)
+        long = _global_staging(self._staging, w.device, _lib.ALGO_BCORR, w.n, max_length, num, _lib.METRIC_MAXABS,
+                               trunc, orth, self._fold())
+        if long:
+            ws = workspace_for(w.device, lib.pp_long_workspace_bytes, _lib.ALGO_BCORR, w.b, w.n, max_length, 0, orth)
+        else:
+            ws = workspace_for(w.device, lib.pp_workspace_bytes, _lib.ALGO_BCORR, w.n, max_length, num, orth)
         cur = torch.cuda.current_stream(w.device)
         for b0, b1, ready in w.launch_plan():
             if ready is not None:
                 cur.wait_event(ready)
+            if long:
+                call(lib.pp_long_best_correlation, "pp_long_best_correlation", w.device,
+                     C.c_void_p(w.ptr + b0 * w.ldx * 8), w.ldx, b1 - b0, w.n, num, max_length, ratio, trunc, orth,
+                     ptr(co), ptr(cq), tb.pmax, ptr(periods[b0:b1]), ptr(powers[b0:b1]),
+                     ptr(None if bases is None else bases[b0:b1]), ptr(status[b0:b1]), ptr(ws), ws.numel(),
+                     stream_ptr(w.device))
+                continue
             call(lib.pp_best_correlation, "pp_best_correlation", w.device, C.c_void_p(w.ptr + b0 * w.ldx * 8), w.ldx,
                  b1 - b0, w.n, num, max_length, ratio, int(self._trunc_to_integer_multiple), int(self._orthogonalize),
                  self._fold(), ptr(co), ptr(cq), tb.pmax, ptr(periods[b0:b1]), ptr(powers[b0:b1]),
@@ -433,11 +513,17 @@ class Periods:
         norms = torch.zeros((w.b, num), dtype=torch.float64, device=dev)
         bases = torch.zeros((w.b, num, n), dtype=torch.float64, device=dev) if return_bases else None
         status = torch.zeros((w.b,), dtype=torch.int32, device=dev)
+        long = _global_staging(self._staging, dev, _lib.ALGO_BFREQ, n, n)
+        ws = workspace_for(dev, lib.pp_long_workspace_bytes, _lib.ALGO_BFREQ, w.b, n, n, 0, 0) if long else None
         for i in range(num):
             mags = torch.abs(torch.fft.rfft(work, win_size, dim=1)).contiguous()
-            call(lib.pp_best_frequency_round, "pp_best_frequency_round", dev, ptr(work), w.b, n, ptr(mags), mags.shape[1],
-                 win_size, int(self._trunc_to_integer_multiple), orth, ptr(co), ptr(cq), tb.pmax, ptr(periods), ptr(norms),
-                 ptr(bases), i, num, ptr(status), stream_ptr(dev))
+            args = (ptr(work), w.b, n, ptr(mags), mags.shape[1], win_size, int(self._trunc_to_integer_multiple), orth,
+                    ptr(co), ptr(cq), tb.pmax, ptr(periods), ptr(norms), ptr(bases), i, num, ptr(status))
+            if long:
+                call(lib.pp_long_best_frequency_round, "pp_long_best_frequency_round", dev, *args, ptr(ws), ws.numel(),
+                     stream_ptr(dev))
+            else:
+                call(lib.pp_best_frequency_round, "pp_best_frequency_round", dev, *args, stream_ptr(dev))
         powers = norms / data_norm[:, None]
         res = BatchResult(_export(w, periods, True), _export(w, powers), _export(w, bases), _export(w, status))
         if w.was_1d:

@@ -72,6 +72,25 @@ def moebius_table(nmax: int) -> np.ndarray:
     return mu
 
 
+def _nontrivial_factor_lists(pmax: int) -> list:
+    """nontrivial_factors(n) for every n in 0..pmax, by a sieve.  Each n receives the same insertion sequence as
+    _divisor_set builds (every divisor i <= sqrt(n) in ascending order, immediately followed by n // i), so set()
+    iterates the divisors in the same order as the per-n expression (load-bearing, SURVEY.md 8a row 3)."""
+    seqs = [[] for _ in range(pmax + 1)]
+    i = 1
+    while i * i <= pmax:
+        for n in range(i * i, pmax + 1, i):
+            seqs[n] += (i, n // i)
+        i += 1
+    out = []
+    for n, seq in enumerate(seqs):
+        s = set(seq)
+        s.discard(1)
+        s.discard(n)
+        out.append(list(s))
+    return out
+
+
 class PeriodTables:
     """CSR tables for all periods 0..pmax, as numpy int32 (host) and cached device tensors."""
 
@@ -80,10 +99,11 @@ class PeriodTables:
         chain_off = np.zeros(self.pmax + 2, dtype=np.int32)
         fac_off = np.zeros(self.pmax + 2, dtype=np.int32)
         chain, fac = [], []
+        factors = _nontrivial_factor_lists(self.pmax)
+        pr = _primes()
         for p in range(self.pmax + 1):
             if p >= 2:
-                fs = nontrivial_factors(p)
-                pr = _primes()
+                fs = factors[p]
                 fac.extend(fs)
                 chain.extend(int(p / f) for f in fs if f in pr)
             chain_off[p + 1] = len(chain)
