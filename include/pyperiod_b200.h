@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PP_ABI_VERSION 6
+#define PP_ABI_VERSION 7
 
 /* sweep metrics */
 #define PP_METRIC_NORM 0   /* ||proj_p|| / sqrt(N)                 Periods.py:221-241, 507-508 */
@@ -297,6 +297,51 @@ int pp_qo_solve_rows(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t
                      const int32_t *dict_rows, const int32_t *n_dict, int32_t pmax, int32_t refine, int32_t rmax,
                      int32_t *n_weights, double *weights, int64_t ldw, double *res, int32_t *status,
                      void *workspace, size_t workspace_bytes, void *stream);
+
+/* ---- QOPeriods on windows that do not fit in shared memory (the "long" path, pp_long_qo.cu) ----------------
+ * pp_qo_fits_on_chip answers, without touching a device, whether the on-chip launch of `kind` fits smem_bytes of
+ * shared memory per block.  It evaluates the plan the launch itself would use:
+ *   PP_QO_KIND_FIND     pp_qo_find_periods (num, rmax, basis; fold_mode decides the hierarchical scratch: pass
+ *                       PP_FOLD_DIRECT for a trunc call, which always folds directly);
+ *   PP_QO_KIND_SOLVE    pp_qo_solve / pp_qo_solve_rows (num = kmax; natural basis), including the choice to read
+ *                       the window in place from global memory;
+ *   PP_QO_KIND_MURESAN  pp_muresan_powers (pmax = max_p; num, rmax, basis, fold_mode are checked but unused).
+ * Windows or periods above 32767 samples never fit (the on-chip find and solve reject them).  1 = fits, 0 = does
+ * not, < 0 = bad arguments.
+ * pp_long_qo_find_periods, pp_long_qo_solve, pp_long_qo_solve_rows and pp_long_muresan_powers take the arguments of
+ * their on-chip namesakes (find: without fold mode, order list, overflow pool and profile buffer; weights are dense,
+ * ldw >= rmax rounded up to 32) plus a workspace, and return the same results for any N.  The windows' residuals
+ * and each window's packed Cholesky factor live in the workspace; batches run in pieces of windows, as many as the
+ * workspace holds (pp_long_qo_workspace_bytes sizes it for a piece of at most half the L2 cache in residuals and at
+ * most factor_budget bytes of factors).  A dictionary holds at most pp_long_qo_max_rows(smem_bytes) rows (the
+ * right-hand side stays in shared memory); above that, and above rmax, a window reports PP_STATUS_TOO_LARGE with the
+ * rows it needs in n_weights.  The calls return after their work is done. */
+#define PP_QO_KIND_FIND 0
+#define PP_QO_KIND_SOLVE 1
+#define PP_QO_KIND_MURESAN 2
+int pp_qo_fits_on_chip(int32_t kind, int32_t N, int32_t pmax, int32_t num, int32_t rmax, int32_t basis,
+                       int32_t fold_mode, int32_t smem_bytes);
+int32_t pp_long_qo_max_rows(int32_t smem_bytes);
+size_t pp_long_qo_workspace_bytes(int32_t kind, int32_t B, int32_t N, int32_t pmax, int32_t num, int32_t rmax,
+                                  int32_t basis, size_t factor_budget);
+int pp_long_qo_find_periods(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t num, double thresh,
+                            int32_t pmin, int32_t pmax, int32_t trunc, int32_t refine, int32_t basis, const int32_t *phi,
+                            int32_t table_pmax, int32_t rmax, uint32_t *periods, double *norms, int32_t *n_periods,
+                            int32_t *dict_q, int32_t *dict_keep, int32_t *n_dict, int32_t *n_weights, double *weights,
+                            int64_t ldw, double *res, int32_t *status, void *workspace, size_t workspace_bytes,
+                            void *stream);
+int pp_long_qo_solve(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t *periods,
+                     const int32_t *nper, int32_t pmax, int32_t refine, const int32_t *phi, int32_t table_pmax,
+                     int32_t rmax, const int32_t *order, int32_t n_order, int32_t *dict_q, int32_t *dict_keep,
+                     int32_t *n_dict, int32_t *n_weights, double *weights, int64_t ldw, const int64_t *weights_off,
+                     double *res, int32_t *status, void *workspace, size_t workspace_bytes, void *stream);
+int pp_long_qo_solve_rows(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t *dict_q,
+                          const int32_t *dict_rows, const int32_t *n_dict, int32_t pmax, int32_t refine, int32_t rmax,
+                          int32_t *n_weights, double *weights, int64_t ldw, double *res, int32_t *status,
+                          void *workspace, size_t workspace_bytes, void *stream);
+int pp_long_muresan_powers(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t max_p, int32_t normalize,
+                           const int32_t *mu, int32_t table_pmax, double *raw, double *pows, int32_t *best,
+                           void *workspace, size_t workspace_bytes, void *stream);
 
 /* ---- QOPeriods.get_periods (QOPeriods.py:719-741 with concatenate_periods :854-887 and
  *      stack_pairwise_gcd_subspaces :889-938), batched ------------------------------------------------------

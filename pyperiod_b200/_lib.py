@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PYPERIOD_B200_LIB selects an alternative build of the same library (kernel tuning experiments)
 LIB_PATH = os.environ.get("PYPERIOD_B200_LIB") or os.path.join(HERE, "libpyperiod_b200.so")
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 METRIC_NORM, METRIC_GAMMA, METRIC_MAXABS, METRIC_IMPOSED = 0, 1, 2, 3
 STATUS_OK, STATUS_NO_PERIOD, STATUS_OVERFLOW, STATUS_SINGULAR, STATUS_GUARD = 0, 1, 2, 3, 4
@@ -21,6 +21,7 @@ BASIS_NATURAL, BASIS_RAMANUJAN = 0, 1
 RAM_FP64, RAM_TF32, RAM_F32COMPAT = 0, 1, 2
 ALGO_SWEEP, ALGO_MBEST, ALGO_S2L, ALGO_BCORR, ALGO_QO, ALGO_RAMANUJAN = 0, 1, 2, 3, 4, 5
 ALGO_PROJECT, ALGO_BFREQ = 6, 7
+QO_KIND_FIND, QO_KIND_SOLVE, QO_KIND_MURESAN = 0, 1, 2
 
 _p = C.c_void_p
 _i32 = C.c_int32
@@ -85,6 +86,16 @@ SIGNATURES = {
                                                _i32, _i32, _p, _p, _sz, _p]),
     "pp_qo_solve_rows": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _p, _i32, _i32, _i32, _p, _p, _i64, _p, _p, _p,
                                    _sz, _p]),
+    "pp_qo_fits_on_chip": (C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32]),
+    "pp_long_qo_max_rows": (_i32, [_i32]),
+    "pp_long_qo_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i32, _i32, _i32, _sz]),
+    "pp_long_qo_find_periods": (C.c_int, [_p, _i64, _i32, _i32, _i32, _f64, _i32, _i32, _i32, _i32, _i32, _p, _i32,
+                                          _i32, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p, _p, _sz, _p]),
+    "pp_long_qo_solve": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _i32, _i32, _p, _i32, _i32, _p, _i32,
+                                   _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
+    "pp_long_qo_solve_rows": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _p, _i32, _i32, _i32, _p, _p, _i64, _p, _p,
+                                        _p, _sz, _p]),
+    "pp_long_muresan_powers": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _p, _i32, _p, _p, _p, _p, _sz, _p]),
 }
 
 _lib = None
@@ -186,6 +197,22 @@ def fits_on_chip(algo: int, n: int, pmax: int, num: int, metric: int, trunc: int
     if rc < 0:
         check(rc, "pp_fits_on_chip")
     return rc == 1
+
+
+def qo_fits_on_chip(kind: int, n: int, pmax: int, num: int, rmax: int, basis: int, fold_mode: int,
+                    smem_bytes: int) -> bool:
+    """Whether the on-chip QO / Muresan launch `kind` (QO_KIND_*) fits `smem_bytes` of shared memory per block
+    (pp_qo_fits_on_chip; no device is touched).  Launches that do not fit run on the global-memory path."""
+    rc = load().pp_qo_fits_on_chip(int(kind), int(n), int(pmax), int(num), int(rmax), int(basis), int(fold_mode),
+                                   int(smem_bytes))
+    if rc < 0:
+        check(rc, "pp_qo_fits_on_chip")
+    return rc == 1
+
+
+def long_qo_max_rows(smem_bytes: int) -> int:
+    """Rows of the largest dictionary the global-memory QO path solves with `smem_bytes` of shared memory."""
+    return int(load().pp_long_qo_max_rows(int(smem_bytes)))
 
 
 def device_info() -> dict:

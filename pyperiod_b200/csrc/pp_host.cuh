@@ -14,6 +14,8 @@ int check_cuda(cudaError_t e, const char* what);
 
 // shared memory of bfreq_round_kernel for windows of N samples (pp_bfreq.cu)
 size_t bfreq_smem_bytes(int N);
+// shared memory of muresan_kernel (pp_muresan.cu)
+size_t muresan_smem_bytes(int N, int max_p);
 
 // fold modes are per-call arguments (include/pyperiod_b200.h)
 static inline int check_fold_mode(int mode) {

@@ -115,6 +115,10 @@ muresan_kernel(const double* __restrict__ x, int64_t ldx, int B, int N, int max_
 
 using namespace pp;
 
+size_t pp::muresan_smem_bytes(int N, int max_p) {
+  return (size_t)(((N + 1) & ~1) + 2 * ((max_p + 1) & ~1) + 2 * kWarps) * 8 + 64;
+}
+
 extern "C" {
 
 int pp_muresan_powers(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t max_p, int32_t normalize,
@@ -124,7 +128,7 @@ int pp_muresan_powers(const double* x, int64_t ldx, int32_t B, int32_t N, int32_
   if (max_p < 2 || max_p > N || table_pmax < max_p - 1) return fail(-1, "need 2 <= max_p <= N and a Moebius table covering max_p - 1%s");
   DeviceFacts f;
   if (int rc = device_facts(f)) return rc;
-  const size_t bytes = (size_t)(((N + 1) & ~1) + 2 * ((max_p + 1) & ~1) + 2 * kWarps) * 8 + 64;
+  const size_t bytes = muresan_smem_bytes(N, max_p);
   if (int rc = prep_kernel(muresan_kernel, bytes, f)) return rc;
   muresan_kernel<<<grid_for(f, bytes, B), kThreads, bytes, (cudaStream_t)stream>>>(x, ldx, B, N, max_p, normalize, mu, raw,
                                                                                   pows, best);

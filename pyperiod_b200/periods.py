@@ -78,12 +78,17 @@ def _global_staging(staging, device, algo, n, pmax, num=0, metric=0, trunc=False
         return True
     if staging == "shared":
         return False
+    return not _lib.fits_on_chip(algo, n, pmax, num, metric, int(bool(trunc)), int(bool(orth)), fold,
+                                 smem_optin(device))
+
+
+def smem_optin(device) -> int:
+    """Opt-in shared memory per block of `device` (cached)."""
     key = str(device)
     if key not in _smem_optin:
         with torch.cuda.device(device):
             _smem_optin[key] = _lib.device_info()["smem_optin_bytes"]
-    return not _lib.fits_on_chip(algo, n, pmax, num, metric, int(bool(trunc)), int(bool(orth)), fold,
-                                 _smem_optin[key])
+    return _smem_optin[key]
 
 
 def _u32(t: torch.Tensor):

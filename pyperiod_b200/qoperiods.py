@@ -21,9 +21,9 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._device import Workspace, call, ptr, stage_windows, stream_ptr, to_host
+from ._device import Workspace, call, ptr, stage_windows, stream_ptr, to_host, workspace_for
 from ._device import RowDownloader
-from .periods import Periods, _export
+from .periods import Periods, _check_staging, _export, smem_optin
 from .tables import get_tables
 
 MAX_ROUNDS = 64  # device-side cap on `num` (the reference's default num = len(data) is "way too many", :377)
@@ -45,6 +45,15 @@ def qo_workspace(lib, dev, n, pmax, num, rmax, basis=_lib.BASIS_NATURAL):
         free, _ = torch.cuda.mem_get_info(dev)
     budget = max(one, int(free * WORKSPACE_FRACTION))
     return Workspace.get(dev, min(full, budget))   # a cached buffer that is already large enough is reused
+
+
+def long_qo_workspace(lib, dev, kind, b, n, pmax, num, rmax, basis=_lib.BASIS_NATURAL):
+    """Workspace of the global-memory QO path: residuals and one Cholesky factor per window of a piece, the factors
+    within the same share of the free device memory as the on-chip launches."""
+    with torch.cuda.device(dev):
+        free, _ = torch.cuda.mem_get_info(dev)
+    return workspace_for(dev, lib.pp_long_qo_workspace_bytes, kind, max(int(b), 1), n, pmax, num, rmax, basis,
+                         int(free * WORKSPACE_FRACTION))
 
 
 def indicator_rows(q: int, n: int, keep) -> np.ndarray:
@@ -174,8 +183,14 @@ def _extract(dev, dq, dk, nd, dq_h, nd_h, weights_flat, ldw, woff):
 class QOPeriods(Periods):
     """Quadratic-program periodicity decomposition (default path), B200-native."""
 
-    def __init__(self, basis_type="natural", trunc_to_integer_multiple=False, orthogonalize=False, device=None):
+    def __init__(self, basis_type="natural", trunc_to_integer_multiple=False, orthogonalize=False, device=None,
+                 staging="auto"):
+        """staging (not in the reference): where a window lives while it is processed, as for Periods.  "shared"
+        stages it in one CTA's shared memory; "global" runs from global memory (csrc/pp_long_qo.cu) for any length;
+        "auto" (default) takes the global-memory path exactly for the launches whose on-chip plan does not fit."""
         super().__init__(trunc_to_integer_multiple, orthogonalize, device=device)
+        _check_staging(staging)
+        self._staging = staging
         self._output = None
         self._basis_type = basis_type
         self._verbose = False
@@ -183,6 +198,13 @@ class QOPeriods(Periods):
         self._window = False
         self._output_bases = None
         self._container = []
+
+    def _long(self, dev, kind, n, pmax, num, rmax, basis=_lib.BASIS_NATURAL, trunc=False) -> bool:
+        """Whether one launch runs on the global-memory path (see `staging`)."""
+        if self._staging != "auto":
+            return self._staging == "global"
+        fold = _lib.FOLD_DIRECT if trunc else self._fold()   # the find kernel folds directly under trunc
+        return not _lib.qo_fits_on_chip(kind, n, pmax, num, rmax, basis, fold, smem_optin(dev))
 
     # ------------------------------------------------------------------ detection
     def find_periods(self, data, num=None, thresh=None, min_length=2, max_length=None, update_weights=True,
@@ -220,6 +242,8 @@ class QOPeriods(Periods):
         # natural basis: more rows than samples is singular by rank, so N rows is the most a factor ever holds;
         # Ramanujan basis: rows <= sum of the periods (no factor is stored, rmax is the capacity of `weights`)
         rows_cap = n if basis == _lib.BASIS_NATURAL else num * int(max_length)
+        if self._staging != "shared":   # dictionaries the global-memory path can hold
+            rows_cap = min(rows_cap, _lib.long_qo_max_rows(smem_optin(w.device)))
         pooled = rmax is None and basis == _lib.BASIS_NATURAL and rows_cap > RMAX_FIRST
         rmax = min(rows_cap, RMAX_FACTOR if pooled else RMAX_FIRST) if rmax is None else int(rmax)
         tb = get_tables(max_length)
@@ -227,10 +251,16 @@ class QOPeriods(Periods):
         phi = tb.phi_device(dev)
         cur = torch.cuda.current_stream(dev)
 
+        trunc = int(self._trunc_to_integer_multiple)
+
         def launch(x_ptr, ldx, count, rmax_l, plan, pool=False, download=False):
             """One pp_qo_find_periods call per piece of `plan` ((first, end, upload event) triples) into one set of
             batch outputs.  pool: the dense weights array keeps RMAX_FIRST columns, larger dictionaries (up to rmax_l
-            rows) put their weights into an overflow pool."""
+            rows) put their weights into an overflow pool.  A launch whose on-chip plan does not fit (or any launch
+            with staging="global") runs whole on the global-memory path, with dense weights."""
+            long = self._long(dev, _lib.QO_KIND_FIND, n, int(max_length), num, rmax_l, basis, trunc)
+            if long:
+                pool = download = False
             rpad = (rmax_l + 31) // 32 * 32
             ldw = min(rpad, (RMAX_FIRST + 31) // 32 * 32) if pool else rpad
             i32 = dict(dtype=torch.int32, device=dev)
@@ -243,6 +273,17 @@ class QOPeriods(Periods):
             slots = max(POOL_MIN_SLOTS, count // POOL_FRACTION) if pool else 0
             o["pool"] = torch.empty((slots, rpad), **f64) if pool else None
             o["pool_slot"] = torch.full((count,), -1, **i32) if pool else None
+            if long:
+                for _, _, ready in plan:
+                    if ready is not None:
+                        cur.wait_event(ready)
+                ws = long_qo_workspace(lib, dev, _lib.QO_KIND_FIND, count, n, int(max_length), num, rmax_l, basis)
+                call(lib.pp_long_qo_find_periods, "pp_long_qo_find_periods", dev, C.c_void_p(x_ptr), ldx, count, n,
+                     num, float(thresh), int(min_length), int(max_length), trunc, int(refine), basis, ptr(phi), tb.pmax,
+                     int(rmax_l), ptr(o["periods"]), ptr(o["norms"]), ptr(o["n_periods"]), ptr(o["dict_q"]),
+                     ptr(o["dict_keep"]), ptr(o["n_dict"]), ptr(o["n_weights"]), ptr(o["weights"]), ldw, ptr(o["res"]),
+                     ptr(o["status"]), ptr(ws), ws.numel(), stream_ptr(dev))
+                return o
             ws = qo_workspace(lib, dev, n, int(max_length), num, rmax_l, basis)
             # host input: the two large results (residuals, dense weights) travel to the host piece by piece while the
             # next piece is being computed
@@ -255,7 +296,7 @@ class QOPeriods(Periods):
                     cur.wait_event(ready)
                 sl = lambda t: ptr(None if t is None else t[b0:b1])
                 call(lib.pp_qo_find_periods, "pp_qo_find_periods", dev, C.c_void_p(x_ptr + b0 * ldx * 8), ldx, b1 - b0,
-                     n, num, float(thresh), int(min_length), int(max_length), int(self._trunc_to_integer_multiple),
+                     n, num, float(thresh), int(min_length), int(max_length), trunc,
                      self._fold(), int(refine), basis, ptr(phi), tb.pmax, int(rmax_l), ptr(None), 0, sl(o["periods"]),
                      sl(o["norms"]), sl(o["n_periods"]), sl(o["dict_q"]), sl(o["dict_keep"]), sl(o["n_dict"]),
                      sl(o["n_weights"]), sl(o["weights"]), ldw, sl(o["res"]), sl(o["status"]), ptr(o["pool"]), slots,
@@ -267,6 +308,8 @@ class QOPeriods(Periods):
                 down.finish()
             return o
 
+        if pooled and self._long(dev, _lib.QO_KIND_FIND, n, int(max_length), num, rmax, basis, trunc):
+            pooled = False   # the global-memory path keeps dense weights
         o = launch(w.ptr, w.ldx, w.b, rmax, w.launch_plan(), pool=pooled,
                    download=w.from_host and w.plan is not None)
         host = o.get("host")
@@ -344,8 +387,13 @@ class QOPeriods(Periods):
         nd, nw, st = (torch.zeros((1,), **i32) for _ in range(3))
         wts = torch.zeros((1, ldw), dtype=torch.float64, device=dev)
         res = torch.empty((1, n), dtype=torch.float64, device=dev)
-        ws = qo_workspace(lib, dev, n, pmax, k, rmax)
-        call(lib.pp_qo_solve, "pp_qo_solve", dev, ptr(w.tensor), w.ldx, 1, n, k, ptr(per), ptr(nper), pmax, int(refine),
+        if self._long(dev, _lib.QO_KIND_SOLVE, n, pmax, k, rmax):
+            ws = long_qo_workspace(lib, dev, _lib.QO_KIND_SOLVE, 1, n, pmax, k, rmax)
+            fn, name = lib.pp_long_qo_solve, "pp_long_qo_solve"
+        else:
+            ws = qo_workspace(lib, dev, n, pmax, k, rmax)
+            fn, name = lib.pp_qo_solve, "pp_qo_solve"
+        call(fn, name, dev, ptr(w.tensor), w.ldx, 1, n, k, ptr(per), ptr(nper), pmax, int(refine),
              ptr(phi), tb.pmax, rmax, ptr(None), 0, ptr(dq), ptr(dk), ptr(nd), ptr(nw), ptr(wts), ldw, ptr(None), ptr(res),
              ptr(st), ptr(ws), ws.numel(), stream_ptr(dev))
         if int(st[0]) != _lib.STATUS_OK:
@@ -378,7 +426,8 @@ class QOPeriods(Periods):
         periods = np.zeros(num, dtype=np.uint32)
         norms = np.zeros(num)
         res, recon, found = x.copy(), None, periods[:0]
-        sweeper = Periods(self._trunc_to_integer_multiple, False, device=w.device, fold_mode=self._fold_mode)
+        sweeper = Periods(self._trunc_to_integer_multiple, False, device=w.device, fold_mode=self._fold_mode,
+                          staging=self._staging)
         for i in range(num):
             if i == 0 or test_function(self, x, recon):
                 _, bp, bv = sweeper.sweep(torch.from_numpy(res).to(w.device), metric="gamma", min_length=int(min_length),
@@ -473,8 +522,13 @@ class QOPeriods(Periods):
         raw = torch.zeros((w.b, max_p), dtype=torch.float64, device=dev)
         pows = torch.zeros((w.b, max_p), dtype=torch.float64, device=dev)
         best = torch.zeros((w.b,), dtype=torch.int32, device=dev)
-        call(lib.pp_muresan_powers, "pp_muresan_powers", dev, ptr(w.tensor), w.ldx, w.b, w.n, max_p, int(bool(normalize)),
-             ptr(tb.mu_device(dev)), tb.pmax, ptr(raw), ptr(pows), ptr(best), stream_ptr(dev))
+        args = (ptr(w.tensor), w.ldx, w.b, w.n, max_p, int(bool(normalize)), ptr(tb.mu_device(dev)), tb.pmax, ptr(raw),
+                ptr(pows), ptr(best))
+        if w.b and self._long(dev, _lib.QO_KIND_MURESAN, w.n, max_p, 1, 2):
+            ws = long_qo_workspace(lib, dev, _lib.QO_KIND_MURESAN, w.b, w.n, max_p, 1, 2)
+            call(lib.pp_long_muresan_powers, "pp_long_muresan_powers", dev, *args, ptr(ws), ws.numel(), stream_ptr(dev))
+        else:
+            call(lib.pp_muresan_powers, "pp_muresan_powers", dev, *args, stream_ptr(dev))
         return w, raw, pows, best, max_p
 
     def get_best_period_orthogonal(self, x, max_p=None, normalize=False, return_powers=False):
@@ -643,8 +697,8 @@ class QOPeriodsWithGCDsExtracted(QOPeriods):
     loop (sweeps, residuals, stop test) is the device loop of QOPeriods; the layout is evaluated on the host
     (CPython set order is part of the reference's output) and the weights are re-solved on the device."""
 
-    def __init__(self, basis_type="natural", trunc_to_integer_multiple=False, device=None):
-        super().__init__(basis_type, trunc_to_integer_multiple, device=device)
+    def __init__(self, basis_type="natural", trunc_to_integer_multiple=False, device=None, staging="auto"):
+        super().__init__(basis_type, trunc_to_integer_multiple, device=device, staging=staging)
 
     def get_subspaces(self, Q, N):
         lay = gcds_extracted_layout(Q)
@@ -683,14 +737,18 @@ class QOPeriodsWithGCDsExtracted(QOPeriods):
             need = max([sum(v if v else int(k) for k, v in lay.items()) for lay in layouts if lay] + [32])
             rmax = min(n, need)
         pmax = int(max(int(lq.max()), 2))
-        ws = qo_workspace(lib, dev, n, pmax, kmax, int(rmax))
+        long = self._long(dev, _lib.QO_KIND_SOLVE, n, pmax, kmax, int(rmax))
+        ws = long_qo_workspace(lib, dev, _lib.QO_KIND_SOLVE, bsz, n, pmax, kmax, int(rmax)) if long else \
+            qo_workspace(lib, dev, n, pmax, kmax, int(rmax))
         t_lq, t_lr, t_ln = (torch.from_numpy(a).to(dev) for a in (lq, lr, ln))
         ldw = (int(rmax) + 31) // 32 * 32
         weights = torch.zeros((bsz, ldw), dtype=torch.float64, device=dev)
         res = torch.empty((bsz, n), dtype=torch.float64, device=dev)
         n_weights = torch.zeros((bsz,), dtype=torch.int32, device=dev)
         status = torch.zeros((bsz,), dtype=torch.int32, device=dev)
-        call(lib.pp_qo_solve_rows, "pp_qo_solve_rows", dev, ptr(w.tensor), w.ldx, bsz, n, kmax, ptr(t_lq), ptr(t_lr),
+        fn, name = (lib.pp_long_qo_solve_rows, "pp_long_qo_solve_rows") if long else (lib.pp_qo_solve_rows,
+                                                                                        "pp_qo_solve_rows")
+        call(fn, name, dev, ptr(w.tensor), w.ldx, bsz, n, kmax, ptr(t_lq), ptr(t_lr),
              ptr(t_ln), pmax, int(refine), int(rmax), ptr(n_weights), ptr(weights), ldw, ptr(res), ptr(status),
              ptr(ws), ws.numel(), stream_ptr(dev))
         out = QOGcdBatchResult(base, layouts, to_host(weights), to_host(n_weights), to_host(res), to_host(status), n=n)

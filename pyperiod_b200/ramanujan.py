@@ -14,7 +14,7 @@ import torch
 from . import _lib
 from ._device import Workspace, call, ptr, stage_windows, stream_ptr, workspace_for
 from .periods import _export
-from .qoperiods import RMAX_FIRST, QOBatchResult, QOPeriods, qo_workspace
+from .qoperiods import RMAX_FIRST, QOBatchResult, QOPeriods, long_qo_workspace, qo_workspace
 from .tables import get_tables
 
 TILE_WINDOWS = 2048      # tf32 / f32_compat: windows whose folds are held at once (7.5 MB per window at qmax = 1365)
@@ -23,13 +23,14 @@ L2_GROUP_WINDOWS = 1024  # fp64 (fused kernel): windows kept L2-resident while e
 
 
 class RamanujanPeriods(QOPeriods):
-    def __init__(self, basis_type="natural", device=None, precision="fp64"):
+    def __init__(self, basis_type="natural", device=None, precision="fp64", staging="auto"):
         """precision (not part of the reference API): "fp64" (FP64 tensor cores, default: the fp64 value of the
         reference's formula), "tf32" (split TF32 contraction on the tcgen05 tensor cores, fp32 accumulation: norms to
         ~1e-5 relative), or "f32_compat" (the reference's own float32 storage and summation order,
         RamanujanPeriods.py:127 and :77-78, reproduced operation by operation: norms equal the reference's to the
-        last float32 bit)."""
-        super().__init__(basis_type, False, False, device=device)
+        last float32 bit).  staging: see QOPeriods; it applies to the solve stage of find_periods_with_weights (the
+        periodogram always runs on chip)."""
+        super().__init__(basis_type, False, False, device=device, staging=staging)
         if precision not in ("fp64", "tf32", "f32_compat"):
             raise ValueError("precision must be 'fp64', 'tf32' or 'f32_compat'")
         self._precision = precision
@@ -139,8 +140,13 @@ class RamanujanPeriods(QOPeriods):
         for order, rmax_l in launches:
             if order.numel() == 0:
                 continue
-            ws = qo_workspace(lib, dev, n, pmax, kmax, rmax_l)
-            call(lib.pp_qo_solve, "pp_qo_solve", dev, ptr(w.tensor), w.ldx, w.b, n, kmax, ptr(periods), ptr(nper), pmax,
+            if self._long(dev, _lib.QO_KIND_SOLVE, n, pmax, kmax, rmax_l):
+                ws = long_qo_workspace(lib, dev, _lib.QO_KIND_SOLVE, int(order.numel()), n, pmax, kmax, rmax_l)
+                fn, name = lib.pp_long_qo_solve, "pp_long_qo_solve"
+            else:
+                ws = qo_workspace(lib, dev, n, pmax, kmax, rmax_l)
+                fn, name = lib.pp_qo_solve, "pp_qo_solve"
+            call(fn, name, dev, ptr(w.tensor), w.ldx, w.b, n, kmax, ptr(periods), ptr(nper), pmax,
                  int(refine), ptr(phi), tb.pmax, int(rmax_l), ptr(order), int(order.numel()), ptr(dict_q), ptr(dict_keep),
                  ptr(n_dict), ptr(n_weights), ptr(weights), 0, ptr(woff), ptr(res), ptr(status), ptr(ws), ws.numel(),
                  stream_ptr(dev))
