@@ -99,7 +99,7 @@ def test_tf32_option_tracks_fp64():
     accumulate); norms within 1e-5 of the fp64 path relative to the largest norm, the thresholded period selection
     is unchanged and so are the weights (the solve stage never sees the periodogram values, only the periods)."""
     from pyperiod_b200 import RamanujanPeriods
-    xb = synth.synth_batch(70, 2048, 61_000)          # 70 windows: a full 64-window tile and a ragged one
+    xb = synth.synth_batch(70, 2048, 61_000)   # one ragged 128-window unit; q <= 400 fits one accumulator tile
     a = RamanujanPeriods().find_periods(xb, 2, 400)
     b = RamanujanPeriods(precision="tf32").find_periods(xb, 2, 400)
     scale = a.max(axis=1, keepdims=True)
@@ -114,6 +114,74 @@ def test_tf32_option_tracks_fp64():
         assert np.array_equal(np.asarray(da["periods"]), np.asarray(db["periods"]))
         assert da["basis_dictionary"] == db["basis_dictionary"]
         np.testing.assert_allclose(db["weights"], da["weights"], rtol=0, atol=1e-12 * np.max(np.abs(da["weights"])))
+
+
+def _planted_cosines(b, n, seed, qmin, qmax, amp):
+    """synth windows, each plus amp * cos(2 pi m / q) for a q drawn from [qmin, qmax]."""
+    rng = np.random.default_rng(seed)
+    xb = synth.synth_batch(b, n, seed)
+    m = np.arange(n)
+    for i in range(b):
+        xb[i] += amp * np.cos(2 * np.pi * m / int(rng.integers(qmin, qmax + 1)))
+    return xb
+
+
+def test_tf32_at_config5_shape_across_tiles(monkeypatch):
+    """precision="tf32" at config 5's shape (N = 4096, q <= 1365) on every tile path of the kernel: with 160 windows
+    per fold tile, 300 windows make two tiles, each a full 128-window unit and a ragged one; q > 512 takes a second
+    512-column accumulator tile.  Strong components at periods in (512, 1365] put the largest norms there.  Norms
+    within 1e-5 of the fp64 path relative to the largest norm, and per q > 512 within 1e-4 of that q's own norm (a
+    dropped or stale accumulator tile cannot hide below the window maximum)."""
+    from pyperiod_b200 import RamanujanPeriods, ramanujan as ram_mod
+    monkeypatch.setattr(ram_mod, "TILE_WINDOWS", 160)
+    xb = _planted_cosines(300, 4096, 64_000, 513, 1365, 4.0)
+    a = RamanujanPeriods().find_periods(xb)
+    b = RamanujanPeriods(precision="tf32").find_periods(xb)
+    assert a.shape == b.shape == (300, 1366)
+    assert np.all(b[:, :2] == 0)
+    scale = a.max(axis=1, keepdims=True)
+    rel = np.abs(a - b) / scale
+    hi = np.abs(a[:, 513:] - b[:, 513:]) / a[:, 513:]
+    print(f"\ntf32: windows with the largest norm above q = 512: {np.mean(a.argmax(axis=1) > 512):.2f}; "
+          f"worst error / largest norm {rel.max():.2g}; worst error / own norm for q > 512 {hi.max():.2g}")
+    assert rel.max() < 1e-5
+    assert hi.max() < 1e-4
+    ra = RamanujanPeriods().find_periods_with_weights(xb, thresh=0.2)
+    rb = RamanujanPeriods(precision="tf32").find_periods_with_weights(xb, thresh=0.2)
+    assert np.array_equal(ra.n_periods, rb.n_periods)
+    assert np.array_equal(ra.periods, rb.periods)
+
+
+def test_fp64_fused_kernel_across_l2_groups(monkeypatch):
+    """The fused fp64 kernel keeps L2_GROUP_WINDOWS windows (rounded up to a multiple of 8) L2-resident while every
+    period passes over them.  Each window's column of the 8-window DMMA product does not depend on the grouping: with
+    groups of 24 windows (24 + 24 + 5) the norms are bit-identical to one group, and so is a hop-framed view."""
+    from pyperiod_b200 import RamanujanPeriods, ramanujan as ram_mod
+    n, hop, count = 2048, 1000, 53
+    stream = synth.synth(n + hop * (count - 1), 65_000)
+    framed = np.lib.stride_tricks.as_strided(stream, (count, n), (hop * 8, 8))   # overlapping windows, ldx < N
+    xb = np.ascontiguousarray(framed)
+    ref = RamanujanPeriods().find_periods(xb)
+    monkeypatch.setattr(ram_mod, "L2_GROUP_WINDOWS", 20)
+    got = RamanujanPeriods().find_periods(xb)
+    assert np.array_equal(got, ref)
+    assert np.array_equal(RamanujanPeriods().find_periods(framed), ref)
+    for b in (0, 26, 52):
+        want = oram.norms_closed_form_f64(xb[b])
+        np.testing.assert_allclose(got[b, 2:], want[2:], rtol=1e-11, atol=0)
+
+
+def test_f32_compat_above_one_accumulator_tile(monkeypatch):
+    """precision="f32_compat" for q up to 700 in a ragged fold tile (3 windows, 2 per tile) against the oracle's
+    float32 emulation of the reference, with the bars of test_f32_compat_reproduces_the_reference_numbers."""
+    from pyperiod_b200 import RamanujanPeriods, ramanujan as ram_mod
+    monkeypatch.setattr(ram_mod, "TILE_WINDOWS", 4)         # f32_compat holds TILE_WINDOWS // 2 windows per tile
+    xb = _planted_cosines(3, 2100, 66_000, 513, 700, 1.0)
+    got = RamanujanPeriods(precision="f32_compat").find_periods(xb, 2, 700)
+    for b in (0, 2):
+        want = oram.find_periods_f32_exact_cq(xb[b], 2, 700)
+        np.testing.assert_allclose(got[b], want, rtol=3e-8)
+        assert np.sum(got[b] == want) >= 0.9 * len(want), int(np.sum(got[b] == want))
 
 
 # ------------------------------------------------------------------ config 5 at its own shape (N = 4096, q <= 1365)
