@@ -415,7 +415,10 @@ __device__ inline int cta_qo_solve_ram(const QoCtx& c, int nfound, double* e_rec
   __syncthreads();
   { const long long now = clock64(); c.t[1] += now - tm; tm = now; }
   RamBasisOp op{ndict, N, c.dict_q, c.dict_rows, c.dict_off, c.tab_off, cq, fold};
-  const int steps = cta_cg_project(op, R, N, c.xs, c.u, r, p, ap, w, c.red, 500);
+  // Budget per pass: R + 16 steps, as gp_kernel.  In exact arithmetic CG ends within rank(G) <= R steps; a fixed
+  // budget below that restarts the pass and discards the Krylov space (1365, 1364, 1024 at N = 4096: about 1040
+  // steps in one pass, no convergence in four passes of 500).
+  const int steps = cta_cg_project(op, R, N, c.xs, c.u, r, p, ap, w, c.red, R + 16);
   __syncthreads();
   if (steps < 0) return PP_STATUS_GUARD;
   for (int i = tid; i < R; i += kThreads) c.wv[i] = w[i];
