@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PYPERIOD_B200_LIB selects an alternative build of the same library (kernel tuning experiments)
 LIB_PATH = os.environ.get("PYPERIOD_B200_LIB") or os.path.join(HERE, "libpyperiod_b200.so")
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 METRIC_NORM, METRIC_GAMMA, METRIC_MAXABS, METRIC_IMPOSED = 0, 1, 2, 3
 STATUS_OK, STATUS_NO_PERIOD, STATUS_OVERFLOW, STATUS_SINGULAR, STATUS_GUARD = 0, 1, 2, 3, 4
@@ -63,6 +63,9 @@ SIGNATURES = {
     "pp_ramanujan_norms_f32compat": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _p, _p, _i32, _i32, _p, _i32, _p, _sz,
                                               _p]),
     "pp_ramanujan_select": (C.c_int, [_p, _i32, _i32, _i32, _f64, _i32, _p, _p, _p]),
+    "pp_ramanujan_fits_on_chip": (C.c_int, [_i32, _i32, _i32, _i32, _i32]),
+    "pp_long_ramanujan_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32]),
+    "pp_long_ramanujan_norms": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _p, _p, _i32, _p, _i32, _p, _sz, _p]),
     "pp_qo_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i32, _i32]),
     "pp_qo_find_periods": (C.c_int, [_p, _i64, _i32, _i32, _i32, _f64, _i32, _i32, _i32, _i32, _i32, _i32, _p, _i32, _i32,
                                      _p, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p, _p, _i32, _p, _p, _sz, _p,
@@ -207,6 +210,15 @@ def qo_fits_on_chip(kind: int, n: int, pmax: int, num: int, rmax: int, basis: in
                                    int(smem_bytes))
     if rc < 0:
         check(rc, "pp_qo_fits_on_chip")
+    return rc == 1
+
+
+def ramanujan_fits_on_chip(mode: int, n: int, qmin: int, qmax: int, smem_bytes: int) -> bool:
+    """Whether the on-chip Ramanujan periodogram of `mode` (RAM_*) fits `smem_bytes` of shared memory per block
+    (pp_ramanujan_fits_on_chip; no device is touched).  fp64 calls that do not fit run on the global-memory path."""
+    rc = load().pp_ramanujan_fits_on_chip(int(mode), int(n), int(qmin), int(qmax), int(smem_bytes))
+    if rc < 0:
+        check(rc, "pp_ramanujan_fits_on_chip")
     return rc == 1
 
 

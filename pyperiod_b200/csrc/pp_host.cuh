@@ -37,6 +37,14 @@ static inline int device_facts(DeviceFacts& f) {
   return 0;
 }
 
+// L2 cache of the current device: the global-memory paths size their pieces from it
+static inline int l2_bytes() {
+  int dev = 0, l2 = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, dev);
+  return l2 > 0 ? l2 : (64 << 20);
+}
+
 // persistent grid: CTAs per SM limited by shared memory (and by kCtasPerSm through registers)
 static inline int grid_for(const DeviceFacts& f, size_t smem_bytes, int B, int max_per_sm = kCtasPerSm) {
   int per_sm = (int)((size_t)(f.smem_optin + 1024) / (smem_bytes + 1024));

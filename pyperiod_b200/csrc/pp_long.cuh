@@ -44,13 +44,6 @@ struct LongWs {
   int* counter = nullptr;    // unit counter of the sweep
 };
 
-static int l2_bytes() {
-  int dev = 0, l2 = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, dev);
-  return l2 > 0 ? l2 : (64 << 20);
-}
-
 // ------------------------------------------------------------------------------------------
 // the sweep: one warp per (window, candidate)
 // ------------------------------------------------------------------------------------------

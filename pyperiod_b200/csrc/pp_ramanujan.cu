@@ -19,31 +19,21 @@
 #include "../../include/pyperiod_b200.h"
 #include "pp_common.cuh"
 #include "pp_host.cuh"
+#include "pp_ram.cuh"
 
 namespace pp {
 
 enum { kModeF64 = PP_RAM_FP64, kModeTf32 = PP_RAM_TF32, kModeF32Compat = PP_RAM_F32COMPAT };
 
 // ------------------------------------------------------------------------------------------
-// dictionary: c_q(n) for all q in [0, qmax], concatenated at offset q (q - 1) / 2 (triangular layout)
+// dictionary: c_q(n) for all q in [0, qmax], concatenated at offset cq_offset(q) = q (q - 1) / 2 (triangular layout)
 // ------------------------------------------------------------------------------------------
-__host__ __device__ inline size_t cq_offset(int q) { return (size_t)q * (q - 1) / 2; }
-
 __global__ void cq_kernel(int qmin, int qmax, const int32_t* __restrict__ mu, const int32_t* __restrict__ phi,
                           double* __restrict__ cq) {
   const int q = qmin + blockIdx.x;
   if (q > qmax) return;
   double* out = cq + cq_offset(q);
-  for (int n = threadIdx.x; n < q; n += blockDim.x) {
-    int a = n, b = q;  // gcd(n, q), gcd(0, q) = q
-    while (a) {
-      const int t = b % a;
-      b = a;
-      a = t;
-    }
-    const int g = b, d = q / g;
-    out[n] = (double)(mu[d] * (phi[q] / phi[d]));
-  }
+  for (int n = threadIdx.x; n < q; n += blockDim.x) out[n] = ramanujan_sum(n, q, mu, phi);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -108,24 +98,6 @@ constexpr int kGemmM = 128;   // rows of H per CTA pass
 constexpr int kGemmN = 64;    // windows per CTA
 constexpr int kGemmK = 32;    // k-chunk staged in shared memory
 constexpr int kLdB = 68;      // padded leading dimension of the staged S chunk (68 mod 16 = 4: conflict-free frags)
-
-// 16-byte asynchronous global -> shared copy; bytes past src_bytes are zero-filled (rows past q, windows past
-// the tile)
-__device__ __forceinline__ void cp_async_16(void* dst_smem, const void* src, int src_bytes) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(dst_smem)), "l"(src), "r"(src_bytes)
-               : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-
-__device__ __forceinline__ void dmma_m8n8k4(double (&c)[2], double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-               : "+d"(c[0]), "+d"(c[1])
-               : "d"(a), "d"(b));
-}
 
 // grid: (ceil(Bt / 64), number of periods).  norms[(b_first + b) * ld_norms + q] = sum_m cnt_q[m] z_m^2.
 __global__ void __launch_bounds__(kThreads, 2)
@@ -877,6 +849,34 @@ size_t pp_ramanujan_workspace_bytes(int32_t N, int32_t qmin, int32_t qmax, int32
   return bytes;
 }
 
+// Shared memory per block of every kernel a mode launches.  The launch below and pp_ramanujan_fits_on_chip both
+// evaluate this plan, so the library's choice between the on-chip and the global-memory periodogram is the launch's.
+struct RamanujanPlan {
+  size_t fused, fold, gemm, umma, compat;
+};
+static RamanujanPlan ramanujan_plan(int N, int qmax) {
+  RamanujanPlan p;
+  FusedPlan fpl;
+  fpl.qmax = qmax;
+  p.fused = fpl.bytes();
+  p.fold = (size_t)kFoldWin * ((N + 1) & ~1) * 8;
+  p.gemm = (size_t)(((qmax + 1) & ~1) + 2 * kGemmK * kLdB + 4 * kGemmN) * 8;
+  UmmaPlan upl;
+  upl.qpad = (qmax + 3 + 31) & ~31;
+  p.umma = upl.bytes();
+  const size_t qe_max = (size_t)((qmax + 1) & ~1);
+  p.compat = (1 + kCompatWin) * qe_max * 8 + kCompatWin * qe_max * 4 + (size_t)kCompatWin * kCompatLeafCap * 4 +
+             2 * (size_t)kCompatLeafCap * 4;
+  return p;
+}
+static bool compat_supports(int N) { return (N + 63) / 64 <= kCompatLeafCap; }
+static bool ramanujan_plan_fits(const RamanujanPlan& p, int mode, int N, size_t smem) {
+  if (mode == kModeF64) return p.fused <= smem;
+  if (p.fold > smem || p.gemm > smem) return false;
+  if (mode == kModeTf32) return p.umma <= smem;
+  return compat_supports(N) && p.compat <= smem;
+}
+
 // norms[b, q] for q in [qmin, qmax] (other entries untouched; the caller zero-fills, RamanujanPeriods.py:71).
 // mu / phi: device int32 tables for 0..table_qmax.  Windows are processed in tiles of `tile_windows`
 // (workspace holds the folds of one tile).
@@ -898,6 +898,7 @@ static int ramanujan_norms_impl(const double* x, int64_t ldx, int32_t B, int32_t
   const size_t rows = (size_t)qmax * (qmax + 1) / 2 - (size_t)qmin * (qmin - 1) / 2;
   size_t off = 0;
   const bool fused = mode == kModeF64;
+  const RamanujanPlan plan = ramanujan_plan(N, qmax);
   double* cq = carve(workspace, workspace_bytes, off, (cq_offset(qmax + 1) + 2) * 8);
   int* next_unit = reinterpret_cast<int*>(carve(workspace, workspace_bytes, off, 256));
   double* S = fused ? nullptr : carve(workspace, workspace_bytes, off, rows * (size_t)ldS * 8);
@@ -907,33 +908,25 @@ static int ramanujan_norms_impl(const double* x, int64_t ldx, int32_t B, int32_t
   cq_kernel<<<qmax - qmin + 1, 128, 0, st>>>(qmin, qmax, mu, phi, cq);
   if (fused) {
     // one launch for the whole batch; tile_windows is the L2 group (windows re-read by every period)
-    FusedPlan pl;
-    pl.qmax = qmax;
-    if (int rc = prep_kernel(ram_fused_kernel, pl.bytes(), f)) return rc;
+    if (int rc = prep_kernel(ram_fused_kernel, plan.fused, f)) return rc;
     const int group_req = tile_windows < B ? tile_windows : B;   // a small batch is one (short) group: no empty units
     const int group = (group_req + kFusedWin - 1) / kFusedWin * kFusedWin;
     const long long units = (long long)(qmax - qmin + 1) * (group / kFusedWin) * ((B + group - 1) / group);
     if (units > 0x7fffffffLL) return fail(-1, "batch too large for one launch%s");
     if (int rc = check_cuda(cudaMemsetAsync(next_unit, 0, sizeof(int), st), "cudaMemsetAsync")) return rc;
-    const int ctas = grid_for(f, pl.bytes(), 0, 2);
+    const int ctas = grid_for(f, plan.fused, 0, 2);
     const int grid = units < ctas ? (int)units : ctas;
-    ram_fused_kernel<<<grid, kThreads, pl.bytes(), st>>>(x, ldx, B, N, qmin, qmax, group, cq, phi, norms, ld_norms,
+    ram_fused_kernel<<<grid, kThreads, plan.fused, st>>>(x, ldx, B, N, qmin, qmax, group, cq, phi, norms, ld_norms,
                                                          next_unit);
     return check_cuda(cudaGetLastError(), "ram_fused_kernel launch");
   }
-  const size_t fold_smem = (size_t)kFoldWin * ((N + 1) & ~1) * 8;
+  const size_t fold_smem = plan.fold, gemm_smem = plan.gemm, compat_smem = plan.compat;
   if (int rc = prep_kernel(fold_all_kernel, fold_smem, f)) return rc;
-  const size_t gemm_smem = (size_t)(((qmax + 1) & ~1) + 2 * kGemmK * kLdB + 4 * kGemmN) * 8;
   if (int rc = prep_kernel(ram_gemm_kernel, gemm_smem, f)) return rc;
-  UmmaPlan upl;
-  upl.qpad = (qmax + 3 + 31) & ~31;
   if (tf32)
-    if (int rc = prep_kernel(ram_umma_tf32_kernel, upl.bytes(), f)) return rc;
-  const size_t qe_max = (size_t)((qmax + 1) & ~1);
-  const size_t compat_smem = (1 + kCompatWin) * qe_max * 8 + kCompatWin * qe_max * 4 +
-                             (size_t)kCompatWin * kCompatLeafCap * 4 + 2 * (size_t)kCompatLeafCap * 4;
+    if (int rc = prep_kernel(ram_umma_tf32_kernel, plan.umma, f)) return rc;
   if (compat) {
-    if ((N + 63) / 64 > kCompatLeafCap) return fail(-1, "float32-compat mode supports N <= 32768%s");
+    if (!compat_supports(N)) return fail(-1, "float32-compat mode supports N <= 32768%s");
     if (int rc = prep_kernel(ram_compat_kernel, compat_smem, f)) return rc;
   }
   for (int b_first = 0; b_first < B; b_first += tile_windows) {
@@ -945,7 +938,7 @@ static int ramanujan_norms_impl(const double* x, int64_t ldx, int32_t B, int32_t
     if (tf32) {
       const int units = (qmax - qmin + 1) * ((b_count + kUW - 1) / kUW);
       if (int rc = check_cuda(cudaMemsetAsync(next_unit, 0, sizeof(int), st), "cudaMemsetAsync")) return rc;
-      ram_umma_tf32_kernel<<<units < f.sm_count ? units : f.sm_count, kThreads, upl.bytes(), st>>>(
+      ram_umma_tf32_kernel<<<units < f.sm_count ? units : f.sm_count, kThreads, plan.umma, st>>>(
           S, ldS, b_first, b_count, N, qmin, qmax, cq, phi, norms, ld_norms, next_unit);
     } else {
       ram_gemm_kernel<<<grid, kThreads, gemm_smem, st>>>(S, ldS, b_first, b_count, N, qmin, qmax, cq, phi, norms,
@@ -980,6 +973,12 @@ int pp_ramanujan_norms_f32compat(const double* x, int64_t ldx, int32_t B, int32_
                                  void* stream) {
   return ramanujan_norms_impl(x, ldx, B, N, qmin, qmax, mu, phi, table_qmax, tile_windows, norms, ld_norms, workspace,
                               workspace_bytes, stream, kModeF32Compat);
+}
+
+int pp_ramanujan_fits_on_chip(int32_t mode, int32_t N, int32_t qmin, int32_t qmax, int32_t smem_bytes) {
+  if (mode != kModeF64 && mode != kModeTf32 && mode != kModeF32Compat) return -1;
+  if (N < 2 || qmin < 1 || qmax < qmin || qmax > N || smem_bytes < 1) return -1;
+  return ramanujan_plan_fits(ramanujan_plan(N, qmax), mode, N, (size_t)smem_bytes) ? 1 : 0;
 }
 
 // periods[b, 0:nper[b]] = ascending q in [0, qlen) with norms[b, q] / |max_q norms[b, q]| > thresh

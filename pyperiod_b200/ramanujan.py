@@ -3,7 +3,8 @@
 `find_periods` is the Ramanujan periodogram: a fold of every period followed by a dense contraction
 with the circulant of Ramanujan sums on the FP64 tensor cores (csrc/pp_ramanujan.cu);
 `find_periods_with_weights` thresholds it on the device and hands the selected periods to the
-QOPeriods solve stage (csrc/pp_qo.cu).  Values are fp64; the reference stores its projection in
+QOPeriods solve stage (csrc/pp_qo.cu).  fp64 periodograms whose on-chip plan does not fit in shared memory run from
+global memory (csrc/pp_long_ram.cu), with the same folds and the same tensor cores.  Values are fp64; the reference stores its projection in
 float32 (RamanujanPeriods.py:127), so agreement with it is bounded by ~1e-7 relative on the norms.
 """
 from __future__ import annotations
@@ -13,7 +14,7 @@ import torch
 
 from . import _lib
 from ._device import Workspace, call, ptr, stage_windows, stream_ptr, workspace_for
-from .periods import _export
+from .periods import _export, smem_optin
 from .qoperiods import RMAX_FIRST, QOBatchResult, QOPeriods, long_qo_workspace, qo_workspace
 from .tables import get_tables
 
@@ -28,8 +29,9 @@ class RamanujanPeriods(QOPeriods):
         reference's formula), "tf32" (split TF32 contraction on the tcgen05 tensor cores, fp32 accumulation: norms to
         ~1e-5 relative), or "f32_compat" (the reference's own float32 storage and summation order,
         RamanujanPeriods.py:127 and :77-78, reproduced operation by operation: norms equal the reference's to the
-        last float32 bit).  staging: see QOPeriods; it applies to the solve stage of find_periods_with_weights (the
-        periodogram always runs on chip)."""
+        last float32 bit).  staging: see QOPeriods; it applies to the solve stage of find_periods_with_weights.  The
+        fp64 periodogram runs on chip when its plan fits in shared memory and from global memory otherwise (the other
+        precisions run on chip only and raise PPError above their limits)."""
         super().__init__(basis_type, False, False, device=device, staging=staging)
         if precision not in ("fp64", "tf32", "f32_compat"):
             raise ValueError("precision must be 'fp64', 'tf32' or 'f32_compat'")
@@ -38,11 +40,22 @@ class RamanujanPeriods(QOPeriods):
         self._k = 0
 
     # ------------------------------------------------------------------ periodogram
-    def _norms_device(self, w, min_length, max_length):
+    def _norms_device(self, w, min_length, max_length, _long=None):
+        """Norms [B, max_length + 1] on the device.  _long (tests): True forces the global-memory fp64 periodogram,
+        None lets the plan decide."""
         lib = _lib.load()
         tb = get_tables(max_length)
         mu, phi = tb.mu_device(w.device), tb.phi_device(w.device)
         mode = {"fp64": _lib.RAM_FP64, "tf32": _lib.RAM_TF32, "f32_compat": _lib.RAM_F32COMPAT}[self._precision]
+        if mode == _lib.RAM_FP64 and _long is None and 1 <= min_length <= max_length <= w.n:
+            _long = not _lib.ramanujan_fits_on_chip(mode, w.n, min_length, max_length, smem_optin(w.device))
+        if mode == _lib.RAM_FP64 and _long:
+            ws = workspace_for(w.device, lib.pp_long_ramanujan_workspace_bytes, w.b, w.n, min_length, max_length)
+            norms = torch.zeros((w.b, max_length + 1), dtype=torch.float64, device=w.device)
+            call(lib.pp_long_ramanujan_norms, "pp_long_ramanujan_norms", w.device, ptr(w.tensor), w.ldx, w.b, w.n,
+                 int(min_length), int(max_length), ptr(mu), ptr(phi), tb.pmax, ptr(norms), max_length + 1, ptr(ws),
+                 ws.numel(), stream_ptr(w.device))
+            return norms
         # fp64: the fused kernel needs no fold storage; `tile` is the group of windows kept L2-resident.  The other
         # modes hold the folds (and products) of one tile in the workspace (7.5 MB per window at qmax = 1365).
         tile = {"fp64": L2_GROUP_WINDOWS, "tf32": TILE_WINDOWS, "f32_compat": TILE_WINDOWS // 2}[self._precision]
