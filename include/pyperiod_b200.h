@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PP_ABI_VERSION 8
+#define PP_ABI_VERSION 9
 
 /* sweep metrics */
 #define PP_METRIC_NORM 0   /* ||proj_p|| / sqrt(N)                 Periods.py:221-241, 507-508 */
@@ -283,6 +283,20 @@ int pp_qo_solve(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t kmax
                 int32_t *n_dict, int32_t *n_weights, double *weights, int64_t ldw, const int64_t *weights_off,
                 double *res, int32_t *status, void *workspace, size_t workspace_bytes, void *stream);
 
+/* The same solve stage for QOPeriods(basis_type="ramanujan") (QOPeriods.py:970-971, 1005-1052): same arguments and
+ * outputs as pp_qo_solve, rows c_q((n - i) mod q), the reconstruction computed by conjugate gradients as in
+ * pp_qo_find_periods with PP_BASIS_RAMANUJAN (weights: the minimum-norm solution; rmax is only the capacity of
+ * `weights`, rows <= sum of the periods).  Periods must lie in [1, pmax].  Status: PP_STATUS_SINGULAR when the
+ * dictionary holds both rows of period 2 (the one exact singularity of this basis, where the reference's LU raises),
+ * PP_STATUS_TOO_LARGE with the rows needed in n_weights when they exceed rmax, PP_STATUS_GUARD when conjugate
+ * gradients do not converge; a window that is not solved gets res = x.  Workspace: pp_qo_workspace_bytes(N, pmax,
+ * kmax, rmax, ctas, PP_BASIS_RAMANUJAN); fit query: PP_QO_KIND_SOLVE_RAMANUJAN. */
+int pp_qo_solve_ramanujan(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t *periods,
+                          const int32_t *nper, int32_t pmax, int32_t refine, const int32_t *phi, int32_t table_pmax,
+                          int32_t rmax, const int32_t *order, int32_t n_order, int32_t *dict_q, int32_t *dict_keep,
+                          int32_t *n_dict, int32_t *n_weights, double *weights, int64_t ldw, const int64_t *weights_off,
+                          double *res, int32_t *status, void *workspace, size_t workspace_bytes, void *stream);
+
 /* rows[b] = rows of the dictionary get_subspaces (QOPeriods.py:830-840) lays out for periods[b, 0:nper[b]):
  * lets the caller size rmax, the ragged weights array and the workspace before pp_qo_solve. */
 int pp_qo_dictionary_rows(int32_t B, int32_t kmax, const int32_t *periods, const int32_t *nper, int32_t pmax,
@@ -303,22 +317,27 @@ int pp_qo_solve_rows(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t
  * shared memory per block.  It evaluates the plan the launch itself would use:
  *   PP_QO_KIND_FIND     pp_qo_find_periods (num, rmax, basis; fold_mode decides the hierarchical scratch: pass
  *                       PP_FOLD_DIRECT for a trunc call, which always folds directly);
- *   PP_QO_KIND_SOLVE    pp_qo_solve / pp_qo_solve_rows (num = kmax; natural basis), including the choice to read
- *                       the window in place from global memory;
+ *   PP_QO_KIND_SOLVE    pp_qo_solve / pp_qo_solve_rows (num = kmax; basis must be PP_BASIS_NATURAL), including the
+ *                       choice to read the window in place from global memory;
+ *   PP_QO_KIND_SOLVE_RAMANUJAN  pp_qo_solve_ramanujan (num = kmax; basis must be PP_BASIS_RAMANUJAN), the same choice;
  *   PP_QO_KIND_MURESAN  pp_muresan_powers (pmax = max_p; num, rmax, basis, fold_mode are checked but unused).
  * Windows or periods above 32767 samples never fit (the on-chip find and solve reject them).  1 = fits, 0 = does
  * not, < 0 = bad arguments.
- * pp_long_qo_find_periods, pp_long_qo_solve, pp_long_qo_solve_rows and pp_long_muresan_powers take the arguments of
- * their on-chip namesakes (find: without fold mode, order list, overflow pool and profile buffer; weights are dense,
- * ldw >= rmax rounded up to 32) plus a workspace, and return the same results for any N.  The windows' residuals
+ * pp_long_qo_find_periods, pp_long_qo_solve, pp_long_qo_solve_ramanujan, pp_long_qo_solve_rows and
+ * pp_long_muresan_powers take the arguments of their on-chip namesakes (find: without fold mode, order list, overflow
+ * pool and profile buffer; weights are dense, ldw >= rmax rounded up to 32) plus a workspace, and return the same
+ * results for any N.  The windows' residuals
  * and each window's packed Cholesky factor live in the workspace; batches run in pieces of windows, as many as the
  * workspace holds (pp_long_qo_workspace_bytes sizes it for a piece of at most half the L2 cache in residuals and at
- * most factor_budget bytes of factors).  A dictionary holds at most pp_long_qo_max_rows(smem_bytes) rows (the
- * right-hand side stays in shared memory); above that, and above rmax, a window reports PP_STATUS_TOO_LARGE with the
+ * most factor_budget bytes of factors; kind and basis as for pp_qo_fits_on_chip, PP_QO_KIND_SOLVE also accepts
+ * PP_BASIS_RAMANUJAN there, which sizes the same per-window state as PP_QO_KIND_SOLVE_RAMANUJAN).  For the Ramanujan
+ * basis the conjugate-gradient vectors take the place of the factor.  A dictionary holds at most
+ * pp_long_qo_max_rows(smem_bytes) rows (the right-hand side stays in shared memory); above that, and above rmax, a window reports PP_STATUS_TOO_LARGE with the
  * rows it needs in n_weights.  The calls return after their work is done. */
 #define PP_QO_KIND_FIND 0
 #define PP_QO_KIND_SOLVE 1
 #define PP_QO_KIND_MURESAN 2
+#define PP_QO_KIND_SOLVE_RAMANUJAN 3
 int pp_qo_fits_on_chip(int32_t kind, int32_t N, int32_t pmax, int32_t num, int32_t rmax, int32_t basis,
                        int32_t fold_mode, int32_t smem_bytes);
 int32_t pp_long_qo_max_rows(int32_t smem_bytes);
@@ -335,6 +354,12 @@ int pp_long_qo_solve(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t
                      int32_t rmax, const int32_t *order, int32_t n_order, int32_t *dict_q, int32_t *dict_keep,
                      int32_t *n_dict, int32_t *n_weights, double *weights, int64_t ldw, const int64_t *weights_off,
                      double *res, int32_t *status, void *workspace, size_t workspace_bytes, void *stream);
+int pp_long_qo_solve_ramanujan(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t *periods,
+                               const int32_t *nper, int32_t pmax, int32_t refine, const int32_t *phi, int32_t table_pmax,
+                               int32_t rmax, const int32_t *order, int32_t n_order, int32_t *dict_q, int32_t *dict_keep,
+                               int32_t *n_dict, int32_t *n_weights, double *weights, int64_t ldw,
+                               const int64_t *weights_off, double *res, int32_t *status, void *workspace,
+                               size_t workspace_bytes, void *stream);
 int pp_long_qo_solve_rows(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t *dict_q,
                           const int32_t *dict_rows, const int32_t *n_dict, int32_t pmax, int32_t refine, int32_t rmax,
                           int32_t *n_weights, double *weights, int64_t ldw, double *res, int32_t *status,

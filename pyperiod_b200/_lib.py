@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PYPERIOD_B200_LIB selects an alternative build of the same library (kernel tuning experiments)
 LIB_PATH = os.environ.get("PYPERIOD_B200_LIB") or os.path.join(HERE, "libpyperiod_b200.so")
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 METRIC_NORM, METRIC_GAMMA, METRIC_MAXABS, METRIC_IMPOSED = 0, 1, 2, 3
 STATUS_OK, STATUS_NO_PERIOD, STATUS_OVERFLOW, STATUS_SINGULAR, STATUS_GUARD = 0, 1, 2, 3, 4
@@ -21,7 +21,7 @@ BASIS_NATURAL, BASIS_RAMANUJAN = 0, 1
 RAM_FP64, RAM_TF32, RAM_F32COMPAT = 0, 1, 2
 ALGO_SWEEP, ALGO_MBEST, ALGO_S2L, ALGO_BCORR, ALGO_QO, ALGO_RAMANUJAN = 0, 1, 2, 3, 4, 5
 ALGO_PROJECT, ALGO_BFREQ = 6, 7
-QO_KIND_FIND, QO_KIND_SOLVE, QO_KIND_MURESAN = 0, 1, 2
+QO_KIND_FIND, QO_KIND_SOLVE, QO_KIND_MURESAN, QO_KIND_SOLVE_RAMANUJAN = 0, 1, 2, 3
 
 _p = C.c_void_p
 _i32 = C.c_int32
@@ -72,6 +72,8 @@ SIGNATURES = {
                                      _p]),
     "pp_qo_solve": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _i32, _i32, _p, _i32, _i32, _p, _i32,
                               _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
+    "pp_qo_solve_ramanujan": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _i32, _i32, _p, _i32, _i32, _p, _i32,
+                                        _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
     "pp_qo_get_periods": (C.c_int, [_i32, _i32, _i32, _i32, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _p, _p]),
     "pp_qo_dictionary_rows": (C.c_int, [_i32, _i32, _p, _p, _i32, _p, _i32, _p, _p]),
     "pp_fits_on_chip": (C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32]),
@@ -96,6 +98,8 @@ SIGNATURES = {
                                           _i32, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p, _p, _sz, _p]),
     "pp_long_qo_solve": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _i32, _i32, _p, _i32, _i32, _p, _i32,
                                    _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
+    "pp_long_qo_solve_ramanujan": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _i32, _i32, _p, _i32, _i32, _p, _i32,
+                                             _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
     "pp_long_qo_solve_rows": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _p, _i32, _i32, _i32, _p, _p, _i64, _p, _p,
                                         _p, _sz, _p]),
     "pp_long_muresan_powers": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _p, _i32, _p, _p, _p, _p, _sz, _p]),

@@ -17,8 +17,9 @@
 //           memory.  Only the right-hand side / weights (wv) and the factorisation's staging area are in shared
 //           memory; wv bounds the dictionary (pp_long_qo_max_rows).  Then qo_commit and the reference's stop test.
 //   The host reads the number of windows still active (4 bytes) once per round and stops at 0.
-// The solve stage alone is one step per window.  Muresan: one warp per (window, q) folds from global memory with
-// muresan_kernel's lane-to-residue mapping and summation order, then one CTA per window runs the Moebius pass.
+// The solve stage alone (either basis) is one step per window.  Muresan: one warp per (window, q) folds from global
+// memory with muresan_kernel's lane-to-residue mapping and summation order, then one CTA per window runs the Moebius
+// pass.
 //
 // Index widths: packed-factor offsets are size_t (pp_chol.cuh), row and sample indices stay below N < 2^31.  The
 // 32767 cap of the on-chip launches comes from the hierarchical fold's 16-bit job descriptors; this path folds
@@ -261,7 +262,9 @@ __global__ void __launch_bounds__(kThreads) long_qo_step_kernel(LongQoArgs a, Qo
   }
 }
 
-// solve stage alone (qo_solve_kernel with the window in place and the factor per window)
+// solve stage alone (qo_solve_kernel with the window in place and the factor -- or, for the Ramanujan basis, the
+// conjugate-gradient vectors -- per window)
+template <int BASIS>
 __global__ void __launch_bounds__(kThreads) long_qo_solve_kernel(LongQoArgs a, int nw, const int32_t* __restrict__ entries,
                                                                  const int32_t* __restrict__ explicit_rows,
                                                                  const int32_t* __restrict__ n_entries, int kmax,
@@ -295,7 +298,7 @@ __global__ void __launch_bounds__(kThreads) long_qo_solve_kernel(LongQoArgs a, i
     }
     __syncthreads();
     double e_recon = 0.0;
-    const int rc = cta_qo_solve(c, nd, &e_recon, explicit_rows != nullptr);
+    const int rc = BASIS == 1 ? cta_qo_solve_ram(c, nd, &e_recon) : cta_qo_solve(c, nd, &e_recon, explicit_rows != nullptr);
     const int ndict = c.misc[0], R = c.misc[1];
     if (rc == PP_STATUS_OK) {
       if (out.dict_q != nullptr)
@@ -475,7 +478,7 @@ int prepare(const DeviceFacts& f, int rmax, bool find, int B, int N, int pmax, i
 int long_qo_solve_launch(const double* x, int64_t ldx, int B, int N, int kmax, const int32_t* entries,
                          const int32_t* explicit_rows, const int32_t* n_entries, int pmax, int refine, const int32_t* phi,
                          int rmax, const int32_t* order, int n_order, QoOut o, void* workspace, size_t workspace_bytes,
-                         cudaStream_t s) {
+                         cudaStream_t s, bool ram = false) {
   const int count = order ? n_order : B;
   if (count == 0) return 0;
   if (count < 0 || count > B) return fail(-1, "bad order list%s");
@@ -484,16 +487,21 @@ int long_qo_solve_launch(const double* x, int64_t ldx, int B, int N, int kmax, c
   if (int rc = device_facts(f)) return rc;
   LongQo q;
   int rmax_eff = 0;
-  if (int rc = prepare(f, rmax, false, count, N, pmax, kmax, false, workspace, workspace_bytes, q, rmax_eff)) return rc;
+  if (int rc = prepare(f, rmax, false, count, N, pmax, kmax, ram, workspace, workspace_bytes, q, rmax_eff)) return rc;
   if (o.weights_off == nullptr && o.ldw < q.pl.rmax)
     return fail(-1, "ldw must be >= rmax rounded up to a multiple of 32 (or pass weights_off)%s");
   const size_t smem = long_qo_smem(q.pl.wv_len());
-  if (int rc = prep_kernel(long_qo_solve_kernel, smem, f)) return rc;
+  if (int rc = ram ? prep_kernel(long_qo_solve_kernel<1>, smem, f) : prep_kernel(long_qo_solve_kernel<0>, smem, f))
+    return rc;
   LongQoArgs a = long_qo_args(q, x, ldx, order, N, kmax, 1, pmax, 0, refine, 0.0, phi);
   for (int b0 = 0; b0 < count; b0 += q.w.piece) {
     const int nw = count - b0 < q.w.piece ? count - b0 : q.w.piece;
     a.b0 = b0;
-    long_qo_solve_kernel<<<step_grid(q.w, nw), kThreads, smem, s>>>(a, nw, entries, explicit_rows, n_entries, kmax, o);
+    if (ram)
+      long_qo_solve_kernel<1><<<step_grid(q.w, nw), kThreads, smem, s>>>(a, nw, entries, nullptr, n_entries, kmax, o);
+    else
+      long_qo_solve_kernel<0><<<step_grid(q.w, nw), kThreads, smem, s>>>(a, nw, entries, explicit_rows, n_entries, kmax,
+                                                                         o);
     if (int rc = check_cuda(cudaGetLastError(), "long_qo_solve_kernel launch")) return rc;
   }
   return check_cuda(cudaStreamSynchronize(s), "cudaStreamSynchronize");
@@ -522,7 +530,8 @@ size_t pp_long_qo_workspace_bytes(int32_t kind, int32_t B, int32_t N, int32_t pm
   if (B < 1 || N < 2 || pmax < 1 || pmax > N || num < 1 || rmax < 2) return 0;
   if (basis != PP_BASIS_NATURAL && basis != PP_BASIS_RAMANUJAN) return 0;
   if (kind == PP_QO_KIND_MURESAN) return (size_t)muresan_piece(B, pmax) * muresan_piece_bytes(pmax) + 256;
-  if (kind != PP_QO_KIND_FIND && kind != PP_QO_KIND_SOLVE) return 0;
+  if (kind != PP_QO_KIND_FIND && kind != PP_QO_KIND_SOLVE && kind != PP_QO_KIND_SOLVE_RAMANUJAN) return 0;
+  if (kind == PP_QO_KIND_SOLVE_RAMANUJAN && basis != PP_BASIS_RAMANUJAN) return 0;
   DeviceFacts f;
   if (device_facts(f)) return 0;
   int rmax_eff = (rmax + kCb - 1) / kCb * kCb;
@@ -603,6 +612,21 @@ int pp_long_qo_solve(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t
   QoOut o{nullptr, nullptr, nullptr, dict_q, dict_keep, n_dict, n_weights, weights, weights_off, ldw, res, status};
   return long_qo_solve_launch(x, ldx, B, N, kmax, periods, nullptr, nper, pmax, refine, phi, rmax, order, n_order, o,
                               workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int pp_long_qo_solve_ramanujan(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t* periods,
+                               const int32_t* nper, int32_t pmax, int32_t refine, const int32_t* phi, int32_t table_pmax,
+                               int32_t rmax, const int32_t* order, int32_t n_order, int32_t* dict_q, int32_t* dict_keep,
+                               int32_t* n_dict, int32_t* n_weights, double* weights, int64_t ldw,
+                               const int64_t* weights_off, double* res, int32_t* status, void* workspace,
+                               size_t workspace_bytes, void* stream) {
+  if (B == 0) return 0;
+  if (int rc = check_qo_long(x, ldx, B, N, kmax, pmax, rmax, phi, table_pmax)) return rc;
+  if (!periods || !nper || !dict_q || !dict_keep || !n_dict || !n_weights || !weights || !status)
+    return fail(-1, "pointers are null%s");
+  QoOut o{nullptr, nullptr, nullptr, dict_q, dict_keep, n_dict, n_weights, weights, weights_off, ldw, res, status};
+  return long_qo_solve_launch(x, ldx, B, N, kmax, periods, nullptr, nper, pmax, refine, phi, rmax, order, n_order, o,
+                              workspace, workspace_bytes, (cudaStream_t)stream, true);
 }
 
 int pp_long_qo_solve_rows(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t* dict_q,

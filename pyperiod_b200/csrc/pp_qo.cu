@@ -9,7 +9,7 @@
 //   -> reconstruction A^T w, residual = data - reconstruction (:517-522), stop test on
 //      rms(reconstruction) (:391).
 // The same solve stage serves RamanujanPeriods.find_periods_with_weights (RamanujanPeriods.py:106-112)
-// through pp_qo_solve.
+// through pp_qo_solve, and the rounds of a custom test_function through pp_qo_solve / pp_qo_solve_ramanujan.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -188,6 +188,8 @@ qo_find_kernel(QoBatch batch, int N, int num, double thresh, int pmin, int pmax,
 // ------------------------------------------------------------------------------------------
 // explicit_rows == nullptr: entries[b, 0:n_entries[b]) are periods in the caller's order, the layout follows
 // get_subspaces.  Otherwise entry k is the period entries[b, k] with its first explicit_rows[b, k] rows (0 = all).
+// BASIS 1 (Ramanujan sums, conjugate gradients in the per-CTA workspace) takes periods only: explicit_rows == nullptr.
+template <int BASIS>   // 0 natural (indicator rows, Cholesky), 1 Ramanujan sums (conjugate gradients)
 __global__ void __launch_bounds__(kThreads, 2)
 qo_solve_kernel(QoBatch batch, int N, int kmax, const int32_t* __restrict__ entries,
                 const int32_t* __restrict__ explicit_rows, const int32_t* __restrict__ n_entries, int pmax, int refine,
@@ -197,7 +199,7 @@ qo_solve_kernel(QoBatch batch, int N, int kmax, const int32_t* __restrict__ entr
   // x0_global: the window is read in place from global memory (L2) instead of being staged -- 32 KB less shared
   // memory, which is what lets dictionaries of up to N rows run two CTAs per SM (the factorisation of one window
   // is a latency-bound chain; the window itself is only read by the right-hand side and the residual)
-  const QoPlan pl = make_qo_plan(N, pmax, kmax, rmax, false, false, x0_global != 0);
+  const QoPlan pl = make_qo_plan(N, pmax, kmax, rmax, false, BASIS == 1, x0_global != 0);
   QoCtx c = make_ctx(smem, pl, N, kmax, refine, phi, ws + (size_t)blockIdx.x * ws_per_cta);
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem + pl.off_bar());
   double* x0 = const_cast<double*>(c.x0);
@@ -233,7 +235,7 @@ qo_solve_kernel(QoBatch batch, int N, int kmax, const int32_t* __restrict__ entr
     }
     __syncthreads();
     double e_recon = 0.0;
-    const int rc = cta_qo_solve(c, nd, &e_recon, explicit_rows != nullptr);
+    const int rc = BASIS == 1 ? cta_qo_solve_ram(c, nd, &e_recon) : cta_qo_solve(c, nd, &e_recon, explicit_rows != nullptr);
     const int ndict = c.misc[0], R = c.misc[1];
     if (rc == PP_STATUS_OK) {
       // norms are the caller's (periodogram values); only layout, weights and residual are produced here
@@ -417,11 +419,11 @@ int pp_qo_find_periods(const double* x, int64_t ldx, int32_t B, int32_t N, int32
 }
 
 // plan of qo_solve_kernel: the window is kept in global memory when that is what makes room for a second CTA per SM
-static QoPlan qo_solve_plan(const DeviceFacts& f, int N, int pmax, int kmax, int rmax, int& x0_global) {
-  QoPlan pl = make_qo_plan(N, pmax, kmax, rmax, false);
+static QoPlan qo_solve_plan(const DeviceFacts& f, int N, int pmax, int kmax, int rmax, int& x0_global, bool ram = false) {
+  QoPlan pl = make_qo_plan(N, pmax, kmax, rmax, false, ram);
   x0_global = 0;
   if (grid_for(f, pl.bytes(), 0, kQoCtasPerSm) < kQoCtasPerSm * f.sm_count) {
-    const QoPlan alt = make_qo_plan(N, pmax, kmax, rmax, false, false, true);
+    const QoPlan alt = make_qo_plan(N, pmax, kmax, rmax, false, ram, true);
     if (grid_for(f, alt.bytes(), 0, kQoCtasPerSm) > grid_for(f, pl.bytes(), 0, kQoCtasPerSm)) {
       pl = alt;
       x0_global = 1;
@@ -433,7 +435,7 @@ static QoPlan qo_solve_plan(const DeviceFacts& f, int N, int pmax, int kmax, int
 static int qo_solve_launch(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t* entries,
                            const int32_t* explicit_rows, const int32_t* n_entries, int32_t pmax, int32_t refine,
                            const int32_t* phi, int32_t rmax, const int32_t* order, int32_t n_order, QoOut o,
-                           void* workspace, size_t workspace_bytes, void* stream) {
+                           void* workspace, size_t workspace_bytes, void* stream, bool ram = false) {
   const int count = order ? n_order : B;
   if (count == 0) return 0;
   if (count < 0 || count > B) return fail(-1, "bad order list%s");
@@ -441,10 +443,11 @@ static int qo_solve_launch(const double* x, int64_t ldx, int32_t B, int32_t N, i
   DeviceFacts f;
   if (int rc = device_facts(f)) return rc;
   int x0_global = 0;
-  const QoPlan pl = qo_solve_plan(f, N, pmax, kmax, rmax, x0_global);
+  const QoPlan pl = qo_solve_plan(f, N, pmax, kmax, rmax, x0_global, ram);
   if (o.weights_off == nullptr && o.ldw < pl.rmax)
     return fail(-1, "ldw must be >= rmax rounded up to a multiple of 32 (or pass weights_off)%s");
-  if (int rc = prep_kernel(qo_solve_kernel, pl.bytes(), f)) return rc;
+  if (int rc = ram ? prep_kernel(qo_solve_kernel<1>, pl.bytes(), f) : prep_kernel(qo_solve_kernel<0>, pl.bytes(), f))
+    return rc;
   size_t off = 0;
   int* next_window = carve_window_counter(workspace, workspace_bytes, off, (cudaStream_t)stream);
   off = (off + 255) & ~(size_t)255;
@@ -453,9 +456,15 @@ static int qo_solve_launch(const double* x, int64_t ldx, int32_t B, int32_t N, i
   const int grid = qo_grid(f, pl, count, workspace_bytes - off);
   if (grid < 1) return fail(-3, "workspace too small for one factor (see pp_qo_workspace_bytes)%s");
   QoBatch batch{x, ldx, count, order};
-  qo_solve_kernel<<<grid, kThreads, pl.bytes(), (cudaStream_t)stream>>>(
-      batch, N, kmax, entries, explicit_rows, n_entries, pmax, refine, phi, pl.rmax, o,
-      reinterpret_cast<unsigned char*>(workspace) + off, pl.ws_per_cta(), next_window, x0_global);
+  unsigned char* ws = reinterpret_cast<unsigned char*>(workspace) + off;
+  if (ram)
+    qo_solve_kernel<1><<<grid, kThreads, pl.bytes(), (cudaStream_t)stream>>>(
+        batch, N, kmax, entries, nullptr, n_entries, pmax, refine, phi, pl.rmax, o, ws, pl.ws_per_cta(), next_window,
+        x0_global);
+  else
+    qo_solve_kernel<0><<<grid, kThreads, pl.bytes(), (cudaStream_t)stream>>>(
+        batch, N, kmax, entries, explicit_rows, n_entries, pmax, refine, phi, pl.rmax, o, ws, pl.ws_per_cta(),
+        next_window, x0_global);
   return check_cuda(cudaGetLastError(), "qo_solve_kernel launch");
 }
 
@@ -471,6 +480,20 @@ int pp_qo_solve(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t kmax
   QoOut o{nullptr, nullptr, nullptr, dict_q, dict_keep, n_dict, n_weights, weights, weights_off, ldw, res, status};
   return qo_solve_launch(x, ldx, B, N, kmax, periods, nullptr, nper, pmax, refine, phi, rmax, order, n_order, o,
                          workspace, workspace_bytes, stream);
+}
+
+int pp_qo_solve_ramanujan(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t* periods,
+                          const int32_t* nper, int32_t pmax, int32_t refine, const int32_t* phi, int32_t table_pmax,
+                          int32_t rmax, const int32_t* order, int32_t n_order, int32_t* dict_q, int32_t* dict_keep,
+                          int32_t* n_dict, int32_t* n_weights, double* weights, int64_t ldw, const int64_t* weights_off,
+                          double* res, int32_t* status, void* workspace, size_t workspace_bytes, void* stream) {
+  if (B == 0) return 0;  // empty batch: nothing to validate or launch
+  if (int rc = qo_check(x, ldx, B, N, kmax, pmax, rmax, phi, table_pmax)) return rc;
+  if (!periods || !nper || !dict_q || !dict_keep || !n_dict || !n_weights || !weights || !status)
+    return fail(-1, "pointers are null%s");
+  QoOut o{nullptr, nullptr, nullptr, dict_q, dict_keep, n_dict, n_weights, weights, weights_off, ldw, res, status};
+  return qo_solve_launch(x, ldx, B, N, kmax, periods, nullptr, nper, pmax, refine, phi, rmax, order, n_order, o,
+                         workspace, workspace_bytes, stream, true);
 }
 
 int pp_qo_solve_rows(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t kmax, const int32_t* dict_q,
@@ -492,8 +515,13 @@ int pp_qo_fits_on_chip(int32_t kind, int32_t N, int32_t pmax, int32_t num, int32
   if (check_fold_mode(fold_mode)) return -1;
   const size_t smem = (size_t)smem_bytes;
   if (kind == PP_QO_KIND_MURESAN) return muresan_smem_bytes(N, pmax) <= smem ? 1 : 0;
-  if (kind != PP_QO_KIND_FIND && kind != PP_QO_KIND_SOLVE) return fail(-1, "unknown kind%s");
-  if (kind == PP_QO_KIND_SOLVE && basis != PP_BASIS_NATURAL) return fail(-1, "the solve stage has the natural basis only%s");
+  if (kind != PP_QO_KIND_FIND && kind != PP_QO_KIND_SOLVE && kind != PP_QO_KIND_SOLVE_RAMANUJAN)
+    return fail(-1, "unknown kind%s");
+  // the solve kinds name their basis: a basis argument that contradicts the kind is rejected
+  if (kind == PP_QO_KIND_SOLVE && basis != PP_BASIS_NATURAL)
+    return fail(-1, "PP_QO_KIND_SOLVE is the natural-basis solve stage (see PP_QO_KIND_SOLVE_RAMANUJAN)%s");
+  if (kind == PP_QO_KIND_SOLVE_RAMANUJAN && basis != PP_BASIS_RAMANUJAN)
+    return fail(-1, "PP_QO_KIND_SOLVE_RAMANUJAN needs basis PP_BASIS_RAMANUJAN%s");
   // qo_check: the hierarchical fold's job descriptors hold N / g and N mod g in 16 bits
   if (N > 32767 || pmax > 32767) return 0;
   if (kind == PP_QO_KIND_FIND) {
@@ -505,7 +533,7 @@ int pp_qo_fits_on_chip(int32_t kind, int32_t N, int32_t pmax, int32_t num, int32
   f.sm_count = 1;
   f.smem_optin = smem_bytes;
   int x0_global = 0;
-  return qo_solve_plan(f, N, pmax, num, rmax, x0_global).bytes() <= smem ? 1 : 0;
+  return qo_solve_plan(f, N, pmax, num, rmax, x0_global, kind == PP_QO_KIND_SOLVE_RAMANUJAN).bytes() <= smem ? 1 : 0;
 }
 
 int pp_qo_dictionary_rows(int32_t B, int32_t kmax, const int32_t* periods, const int32_t* nper, int32_t pmax,

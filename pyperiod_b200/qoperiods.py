@@ -6,7 +6,8 @@ one persistent kernel per batch (csrc/pp_qo.cu): gamma sweep -> dictionary layou
 (B, N) batch returns a QOBatchResult whose `.window(b)` rebuilds that pair for one window.
 
 Supported: `_orthogonalize=False`, `update_weights=True`, `basis_type` "natural" (default) and "ramanujan"
-(QOPeriods.py:970-971, 1005-1052), the default `test_function` on the device and a custom one for 1-D input.
+(QOPeriods.py:970-971, 1005-1052), the default `test_function` on the device and a custom one (a host callable
+between batched rounds, 1-D or (B, N), either basis).
 `_orthogonalize=True` is dead in the reference (best_base is None) and `update_weights=False` raises OverflowError
 there under numpy 2: both raise NotImplementedError here instead of silently doing something else.
 Deviation from the reference: the stray `print(nonzero_periods)` at QOPeriods.py:488 is not reproduced.
@@ -23,7 +24,7 @@ import torch
 from . import _lib
 from ._device import Workspace, call, ptr, stage_windows, stream_ptr, to_host, workspace_for
 from ._device import RowDownloader
-from .periods import Periods, _check_staging, _export, smem_optin
+from .periods import Periods, _check_staging, _export, _u32, smem_optin
 from .tables import get_tables
 
 MAX_ROUNDS = 64  # device-side cap on `num` (the reference's default num = len(data) is "way too many", :377)
@@ -213,7 +214,11 @@ class QOPeriods(Periods):
 
         Not in the reference: rmax (dictionary rows the first launch holds factors for; windows that outgrow it are
         re-run with room for N rows, so no window is dropped), refine (steps of iterative refinement of the normal
-        equations, default 1), return_res."""
+        equations, default 1), return_res.
+
+        test_function(self, data, reconstruction) (QOPeriods.py:388-391, 418) replaces the default stop test for 1-D
+        input and batches alike; it is called with numpy 1-D arrays once per window and round, round-major and in
+        ascending window order within a round (a stateful test sees that order)."""
         test_function = kwargs.pop("test_function", None)
         if kwargs:
             raise TypeError(f"unexpected arguments {sorted(kwargs)}")
@@ -223,8 +228,8 @@ class QOPeriods(Periods):
         if self._basis_type not in ("natural", "ramanujan"):
             raise ValueError("basis_type must be 'natural' or 'ramanujan'")
         if test_function is not None:
-            return self._find_periods_custom_test(data, num, thresh, min_length, max_length, test_function,
-                                                  rmax=rmax, refine=refine)
+            return self._find_periods_custom_test(data, num, min_length, max_length, test_function, rmax, refine,
+                                                  return_res)
         basis = _lib.BASIS_RAMANUJAN if self._basis_type == "ramanujan" else _lib.BASIS_NATURAL
         lib = _lib.load()
         w = stage_windows(data, self._device, pipeline=True)
@@ -363,94 +368,142 @@ class QOPeriods(Periods):
         return out
 
     # ------------------------------------------------------------------ custom stop test (QOPeriods.py:388-391, 418)
-    def _solve_periods(self, w, found, refine):
-        """get_subspaces + solve_quadratic for the periods `found` (in found order) of the 1-D window `w`, on the device
-        (pp_qo_solve).  Returns (layout, weights, residual) as numpy; raises LinAlgError where the reference does."""
+    def _find_periods_custom_test(self, data, num, min_length, max_length, test_function, rmax, refine, return_res):
+        """The loop of QOPeriods.py:417-594 with a caller-supplied `test_function(self, data, reconstruction)` for B >= 1
+        windows and both bases.  A host callable decides after every round, so the rounds are separate launches; each
+        round serves every window still running:
+          1. one gamma sweep of the active residuals (Periods.sweep with this instance's fold mode and staging);
+          2. one pp_qo_dictionary_rows of every active window's periods, which sizes step 3;
+          3. one solve of those periods against the original data (pp_qo_solve / pp_qo_solve_ramanujan, or their
+             global-memory namesakes where the launch does not fit on chip): windows above RMAX_FIRST rows (or all
+             of them, with an explicit rmax) go to a second launch sized for the largest one;
+          4. one download of the solved windows' residuals, from which the reconstructions data - res are formed;
+          5. test_function(self, x_b, recon_b) with numpy 1-D arrays for each solved window, in ascending window
+             order (the calls are round-major: every window's test of round i comes before any of round i + 1).
+        Per window: zero input gives the reference's canned result (:394-406); a failed solve (status SINGULAR,
+        TOO_LARGE or GUARD) ends the window with the previous round's outputs (:552-559); False from the test ends it
+        with the weights of all periods found and the last period not reported (:560-594)."""
         lib = _lib.load()
-        dev, n = w.device, w.n
-        k = len(found)
-        i32 = dict(dtype=torch.int32, device=dev)
-        per = torch.tensor([list(map(int, found))], **i32)
-        nper = torch.tensor([k], **i32)
-        pmax = int(max(max(map(int, found)), 2))
-        tb = get_tables(pmax)
-        phi = tb.phi_device(dev)
-        rows = torch.zeros((1,), **i32)
-        call(lib.pp_qo_dictionary_rows, "pp_qo_dictionary_rows", dev, 1, k, ptr(per), ptr(nper), pmax, ptr(phi), tb.pmax,
-             ptr(rows), stream_ptr(dev))
-        r = int(rows[0])
-        if r > n:
-            raise np.linalg.LinAlgError("Singular matrix")   # more rows than samples
-        rmax = max(r, 32)
-        ldw = (rmax + 31) // 32 * 32
-        dq, dk = torch.zeros((1, k), **i32), torch.zeros((1, k), **i32)
-        nd, nw, st = (torch.zeros((1,), **i32) for _ in range(3))
-        wts = torch.zeros((1, ldw), dtype=torch.float64, device=dev)
-        res = torch.empty((1, n), dtype=torch.float64, device=dev)
-        if self._long(dev, _lib.QO_KIND_SOLVE, n, pmax, k, rmax):
-            ws = long_qo_workspace(lib, dev, _lib.QO_KIND_SOLVE, 1, n, pmax, k, rmax)
-            fn, name = lib.pp_long_qo_solve, "pp_long_qo_solve"
-        else:
-            ws = qo_workspace(lib, dev, n, pmax, k, rmax)
-            fn, name = lib.pp_qo_solve, "pp_qo_solve"
-        call(fn, name, dev, ptr(w.tensor), w.ldx, 1, n, k, ptr(per), ptr(nper), pmax, int(refine),
-             ptr(phi), tb.pmax, rmax, ptr(None), 0, ptr(dq), ptr(dk), ptr(nd), ptr(nw), ptr(wts), ldw, ptr(None), ptr(res),
-             ptr(st), ptr(ws), ws.numel(), stream_ptr(dev))
-        if int(st[0]) != _lib.STATUS_OK:
-            raise np.linalg.LinAlgError("Singular matrix")
-        m = int(nd[0])
-        layout = {str(int(q)): int(c) for q, c in zip(dq[0, :m].tolist(), dk[0, :m].tolist())}
-        return layout, wts[0, : int(nw[0])].cpu().numpy(), res[0].cpu().numpy()
-
-    def _find_periods_custom_test(self, data, num, thresh, min_length, max_length, test_function, rmax=None, refine=1):
-        """The loop of QOPeriods.py:417-594 with a caller-supplied `test_function(self, data, reconstruction)`: a host
-        callable decides after every round, so the rounds are separate launches (gamma sweep of the residual, then
-        dictionary + normal equations of all periods found so far against the original data).  1-D input, natural
-        basis."""
-        if self._basis_type != "natural":
-            raise NotImplementedError("a custom test_function is supported with basis_type='natural'")
+        ram = self._basis_type == "ramanujan"
+        basis = _lib.BASIS_RAMANUJAN if ram else _lib.BASIS_NATURAL
+        kind = _lib.QO_KIND_SOLVE_RAMANUJAN if ram else _lib.QO_KIND_SOLVE
+        solvers = {(False, False): "pp_qo_solve", (False, True): "pp_qo_solve_ramanujan",
+                   (True, False): "pp_long_qo_solve", (True, True): "pp_long_qo_solve_ramanujan"}
         w = stage_windows(data, self._device)
-        if not w.was_1d:
-            raise NotImplementedError("a custom test_function is a host callable: pass one 1-D signal")
-        n = w.n
-        x = to_host(w.tensor)[0]
+        n, bsz, dev = w.n, w.b, w.device
         if max_length is None:
             max_length = int(np.floor(n / 3))
         num = n if num is None else int(num)
-        if np.sum(np.abs(x)) <= 1e-16:   # QOPeriods.py:394-406
-            out = {"periods": np.array([1]), "norms": np.array([0]), "subspaces": np.ones((1, n)),
-                   "weights": np.array([0]), "basis_dictionary": {"1": n}}
-            self._output = out
-            return out, np.zeros(n)
-        out = {"periods": [], "norms": [], "subspaces": [], "weights": [], "basis_dictionary": {}}
-        periods = np.zeros(num, dtype=np.uint32)
-        norms = np.zeros(num)
-        res, recon, found = x.copy(), None, periods[:0]
-        sweeper = Periods(self._trunc_to_integer_multiple, False, device=w.device, fold_mode=self._fold_mode,
+        i32 = dict(dtype=torch.int32, device=dev)
+        xs = torch.as_strided(w.tensor, (bsz, n), (w.ldx, 1))
+        x_host = to_host(xs) if bsz else np.zeros((0, n))
+        zero = np.sum(np.abs(x_host), axis=1) <= 1e-16   # QOPeriods.py:394-406
+        # per-window outputs: the small ones on the host, residuals and (ragged) weights on the device
+        found = np.zeros((bsz, num), np.int32)           # periods in found order
+        nfound = np.zeros(bsz, np.int32)
+        norms = np.zeros((bsz, num))                     # by round, as the reference indexes them (:476-477)
+        periods = np.zeros((bsz, num), np.int32)
+        n_periods = np.zeros(bsz, np.int32)
+        dict_q, dict_keep = np.zeros((bsz, num), np.int32), np.zeros((bsz, num), np.int32)
+        n_dict, n_weights = np.zeros(bsz, np.int32), np.zeros(bsz, np.int32)
+        status = np.where(zero, _lib.STATUS_ZERO_INPUT, _lib.STATUS_OK).astype(np.int32)
+        woff = np.zeros(bsz, np.int64)
+        weights = torch.zeros((1,), dtype=torch.float64, device=dev)
+        res = xs.clone()
+        res[torch.from_numpy(np.flatnonzero(zero)).to(dev)] = 0.0
+        sweeper = Periods(self._trunc_to_integer_multiple, False, device=dev, fold_mode=self._fold_mode,
                           staging=self._staging)
+        active = np.flatnonzero(~zero)
         for i in range(num):
-            if i == 0 or test_function(self, x, recon):
-                _, bp, bv = sweeper.sweep(torch.from_numpy(res).to(w.device), metric="gamma", min_length=int(min_length),
-                                          max_length=int(max_length))
-                periods[i], norms[i] = int(bp[0]), float(bv[0])
-                found = periods[periods > 0]
-                try:
-                    layout, wts, res = self._solve_periods(w, found, refine)
-                except np.linalg.LinAlgError:   # QOPeriods.py:552-559: keep the previous round's outputs
-                    break
-                recon = x - res
-                out = {"periods": found, "norms": norms[: len(found)],
-                       "subspaces": build_subspaces([int(q) for q in layout], list(layout.values()), n),
-                       "weights": wts, "basis_dictionary": layout}
-                self._output_bases = out
-            else:   # QOPeriods.py:560-594: weights of all periods, the last period not reported
-                layout, wts, _ = self._solve_periods(w, found, refine)
-                out = {"periods": found[:-1], "norms": norms[: len(found) - 1],
-                       "subspaces": build_subspaces([int(q) for q in layout], list(layout.values()), n),
-                       "weights": wts, "basis_dictionary": layout}
+            if not active.size:
                 break
-        self._output = out
-        return out, res
+            act_d = torch.from_numpy(active).to(dev)
+            _, bp, bv = sweeper.sweep(res[act_d], metric="gamma", min_length=int(min_length), max_length=int(max_length))
+            bp, bv = bp.cpu().numpy(), bv.cpu().numpy()
+            norms[active, i] = bv
+            got = active[bp > 0]
+            found[got, nfound[got]] = bp[bp > 0]
+            nfound[got] += 1
+            kmax = max(int(nfound[active].max()), 1)
+            pmax = max(int(found[active, :kmax].max()), 2)
+            tb = get_tables(pmax)
+            phi = tb.phi_device(dev)
+            nper_h = np.zeros(bsz, np.int32)
+            nper_h[active] = nfound[active]
+            per_d = torch.from_numpy(np.ascontiguousarray(found[:, :kmax])).to(dev)
+            nper_d = torch.from_numpy(nper_h).to(dev)
+            rows_d = torch.zeros((bsz,), **i32)
+            call(lib.pp_qo_dictionary_rows, "pp_qo_dictionary_rows", dev, bsz, kmax, ptr(per_d), ptr(nper_d), pmax,
+                 ptr(phi), tb.pmax, ptr(rows_d), stream_ptr(dev))
+            rows = rows_d.cpu().numpy().astype(np.int64)
+            # weights storage for the dictionaries that can be solved (natural basis: more rows than samples is
+            # singular by rank)
+            kept = rows if ram else np.where(rows <= n, rows, 0)
+            woff_r = np.cumsum(kept) - kept
+            wts_r = torch.zeros((max(int(kept.sum()), 1),), dtype=torch.float64, device=dev)
+            dq_r, dk_r = torch.zeros((bsz, kmax), **i32), torch.zeros((bsz, kmax), **i32)
+            nd_r, nw_r, st_r = (torch.zeros((bsz,), **i32) for _ in range(3))
+            res_r = torch.empty((bsz, n), dtype=torch.float64, device=dev)
+            if rmax is not None:
+                launches = [(active, int(rmax))]
+            else:
+                big = kept[active] > RMAX_FIRST
+                launches = [(active[~big], min(RMAX_FIRST, max(int(kept[active[~big]].max(initial=0)), 32))),
+                            (active[big], int(kept[active[big]].max(initial=0)))]
+            for order, rmax_l in launches:
+                if not order.size:
+                    continue
+                long = self._long(dev, kind, n, pmax, kmax, rmax_l, basis)
+                ws = long_qo_workspace(lib, dev, kind, order.size, n, pmax, kmax, rmax_l, basis) if long else \
+                    qo_workspace(lib, dev, n, pmax, kmax, rmax_l, basis)
+                name = solvers[(long, ram)]
+                order_d = torch.from_numpy(order.astype(np.int32)).to(dev)
+                call(getattr(lib, name), name, dev, ptr(w.tensor), w.ldx, bsz, n, kmax, ptr(per_d), ptr(nper_d), pmax,
+                     int(refine), ptr(phi), tb.pmax, rmax_l, ptr(order_d), int(order.size), ptr(dq_r), ptr(dk_r),
+                     ptr(nd_r), ptr(nw_r), ptr(wts_r), 0, ptr(torch.from_numpy(woff_r).to(dev)), ptr(res_r), ptr(st_r),
+                     ptr(ws), ws.numel(), stream_ptr(dev))
+            st = st_r.cpu().numpy()
+            ok = active[st[active] == _lib.STATUS_OK]
+            failed = active[st[active] != _lib.STATUS_OK]
+            status[failed] = st[failed]                 # LinAlgError in the reference: previous outputs stay (:552-559)
+            if ok.size:
+                periods[ok] = found[ok]
+                n_periods[ok] = nfound[ok]
+                dict_q[ok, :kmax] = dq_r.cpu().numpy()[ok]
+                dict_keep[ok, :kmax] = dk_r.cpu().numpy()[ok]
+                n_dict[ok] = nd_r.cpu().numpy()[ok]
+                ok_d = torch.from_numpy(ok).to(dev)
+                res[ok_d] = res_r[ok_d]
+                # ragged weights: this round's for the solved windows, the kept ones for every other window
+                nw = n_weights.astype(np.int64)
+                nw[ok] = nw_r.cpu().numpy()[ok]
+                src = woff.copy()
+                src[ok] = weights.numel() + woff_r[ok]
+                off = np.cumsum(nw) - nw
+                idx = np.repeat(src - off, nw) + np.arange(int(nw.sum()))
+                weights = torch.cat([weights, wts_r])[torch.from_numpy(idx).to(dev)]
+                n_weights, woff = nw.astype(np.int32), off
+            active = ok
+            if i + 1 >= num or not ok.size:
+                break
+            recon = x_host[ok] - to_host(res[ok_d])
+            go = np.array([bool(test_function(self, x_host[b], recon[j])) for j, b in enumerate(ok)])
+            stop = ok[~go]
+            n_periods[stop] = np.maximum(nfound[stop] - 1, 0)   # weights of all periods, the last not reported (:560-594)
+            active = ok[go]
+        host = w.from_host
+        dv = (lambda a: a) if host else (lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev))
+        out = QOBatchResult(periods.view(np.uint32) if host else _u32(dv(periods)), dv(norms), dv(n_periods),
+                            dv(dict_q), dv(dict_keep), dv(n_dict), to_host(weights) if host else weights, dv(n_weights),
+                            (to_host(res) if host else res) if return_res else None, dv(status), n=n,
+                            weights_off=dv(woff), basis=self._basis_type)
+        if w.was_1d:
+            if int(out.status[0]) == _lib.STATUS_TOO_LARGE:
+                raise ValueError("dictionary has more rows than rmax; pass a larger rmax")
+            pair = out.window(0)
+            self._output = self._output_bases = pair[0]
+            return pair
+        return out
 
     # ------------------------------------------------------------------ extraction (QOPeriods.py:719-741)
     def get_periods(self, weights, dictionary=None, decomp_type="row reduction"):
