@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PP_ABI_VERSION 9
+#define PP_ABI_VERSION 10
 
 /* sweep metrics */
 #define PP_METRIC_NORM 0   /* ||proj_p|| / sqrt(N)                 Periods.py:221-241, 507-508 */
@@ -451,6 +451,34 @@ size_t pp_long_ramanujan_workspace_bytes(int32_t B, int32_t N, int32_t qmin, int
 int pp_long_ramanujan_norms(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t qmin, int32_t qmax,
                             const int32_t *mu, const int32_t *phi, int32_t table_qmax, double *norms, int32_t ld_norms,
                             void *workspace, size_t workspace_bytes, void *stream);
+
+/* ---- the Ramanujan periodogram in divisor form (pp_ram_divisor.cu) ---------------------------------------------
+ * The same fp64 quantity as pp_ramanujan_norms / pp_long_ramanujan_norms, computed without the dense contraction:
+ * c_q(n) = sum_{d | gcd(n, q)} mu(q/d) d turns H S_q into an in-place product over the distinct primes p of q,
+ *     z = (q / rad(q)) prod_p (p I - A_p) S_q,     (A_p v)_m = sum_{k < p} v[(m + k q / p) mod q],
+ * and norms[b, q] = (q / phi(q)^2)^2 sum_m cnt_q[m] z_m^2.  Work per (window, period): the fold (N adds, summed in
+ * increasing n per residue as the sweeps do) plus about 2 omega(q) q; no dense product, so the norms differ from the
+ * dense path's by rounding only (rtol 1e-11).  Each (window, period) is computed by one warp or one CTA with
+ * fixed-order sums: two runs are bit-identical.
+ * staging: PP_STAGING_SHARED stages each window in shared memory once and spreads its periods over the CTA's warps
+ * (fails with -1 when that plan does not fit the device); PP_STAGING_GLOBAL folds every (window, period) unit from
+ * global memory (L2), any N; PP_STAGING_AUTO takes SHARED when the plan fits.
+ * pp_ramanujan_divisor_fits_on_chip answers, without touching a device, whether the SHARED plan fits smem_bytes of
+ * shared memory per block: 1 / 0, -1 on bad arguments.
+ * pp_ramanujan_divisor_workspace_bytes: a 256-byte unit counter plus, when qmax > 8192, one scratch slice of
+ * qmax + ceil(qmax / 2) doubles (+ 1, rounded to even) per CTA of the global-memory launch (at most 296), i.e. at most
+ *     256 + 296 * 8 * (qmax + ceil(qmax / 2) + 2) bytes  (O(CTAs x qmax), nothing grows with qmax^2);
+ * 0 on bad arguments.  A smaller workspace lowers the number of CTAs the global-memory launch uses.
+ * spf / phi: device int32 tables (smallest prime factor, totient) for 0..table_qmax.  Only columns qmin..qmax of
+ * norms[B, ld_norms] are written. */
+#define PP_STAGING_AUTO 0
+#define PP_STAGING_SHARED 1
+#define PP_STAGING_GLOBAL 2
+int pp_ramanujan_divisor_fits_on_chip(int32_t N, int32_t qmin, int32_t qmax, int32_t smem_bytes);
+size_t pp_ramanujan_divisor_workspace_bytes(int32_t B, int32_t N, int32_t qmin, int32_t qmax);
+int pp_ramanujan_norms_divisor(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t qmin, int32_t qmax,
+                               const int32_t *spf, const int32_t *phi, int32_t table_qmax, int32_t staging,
+                               double *norms, int32_t ld_norms, void *workspace, size_t workspace_bytes, void *stream);
 
 /* periods[b, 0:nper[b]] = ascending q in [0, qlen) with norms[b,q] / |max_q norms[b,q]| > thresh
  * (RamanujanPeriods.py:97-101); nper[b] may exceed kmax, only the first kmax are stored. */

@@ -12,13 +12,14 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PYPERIOD_B200_LIB selects an alternative build of the same library (kernel tuning experiments)
 LIB_PATH = os.environ.get("PYPERIOD_B200_LIB") or os.path.join(HERE, "libpyperiod_b200.so")
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 METRIC_NORM, METRIC_GAMMA, METRIC_MAXABS, METRIC_IMPOSED = 0, 1, 2, 3
 STATUS_OK, STATUS_NO_PERIOD, STATUS_OVERFLOW, STATUS_SINGULAR, STATUS_GUARD = 0, 1, 2, 3, 4
 STATUS_TOO_LARGE, STATUS_ZERO_INPUT = 5, 6
 BASIS_NATURAL, BASIS_RAMANUJAN = 0, 1
 RAM_FP64, RAM_TF32, RAM_F32COMPAT = 0, 1, 2
+STAGING_AUTO, STAGING_SHARED, STAGING_GLOBAL = 0, 1, 2
 ALGO_SWEEP, ALGO_MBEST, ALGO_S2L, ALGO_BCORR, ALGO_QO, ALGO_RAMANUJAN = 0, 1, 2, 3, 4, 5
 ALGO_PROJECT, ALGO_BFREQ = 6, 7
 QO_KIND_FIND, QO_KIND_SOLVE, QO_KIND_MURESAN, QO_KIND_SOLVE_RAMANUJAN = 0, 1, 2, 3
@@ -66,6 +67,10 @@ SIGNATURES = {
     "pp_ramanujan_fits_on_chip": (C.c_int, [_i32, _i32, _i32, _i32, _i32]),
     "pp_long_ramanujan_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32]),
     "pp_long_ramanujan_norms": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _p, _p, _i32, _p, _i32, _p, _sz, _p]),
+    "pp_ramanujan_divisor_fits_on_chip": (C.c_int, [_i32, _i32, _i32, _i32]),
+    "pp_ramanujan_divisor_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32]),
+    "pp_ramanujan_norms_divisor": (C.c_int, [_p, _i64, _i32, _i32, _i32, _i32, _p, _p, _i32, _i32, _p, _i32, _p, _sz,
+                                             _p]),
     "pp_qo_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i32, _i32]),
     "pp_qo_find_periods": (C.c_int, [_p, _i64, _i32, _i32, _i32, _f64, _i32, _i32, _i32, _i32, _i32, _i32, _p, _i32, _i32,
                                      _p, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p, _p, _i32, _p, _p, _sz, _p,
@@ -223,6 +228,15 @@ def ramanujan_fits_on_chip(mode: int, n: int, qmin: int, qmax: int, smem_bytes: 
     rc = load().pp_ramanujan_fits_on_chip(int(mode), int(n), int(qmin), int(qmax), int(smem_bytes))
     if rc < 0:
         check(rc, "pp_ramanujan_fits_on_chip")
+    return rc == 1
+
+
+def ramanujan_divisor_fits_on_chip(n: int, qmin: int, qmax: int, smem_bytes: int) -> bool:
+    """Whether the on-chip divisor-form Ramanujan periodogram fits `smem_bytes` of shared memory per block
+    (pp_ramanujan_divisor_fits_on_chip; no device is touched).  Calls that do not fit run from global memory."""
+    rc = load().pp_ramanujan_divisor_fits_on_chip(int(n), int(qmin), int(qmax), int(smem_bytes))
+    if rc < 0:
+        check(rc, "pp_ramanujan_divisor_fits_on_chip")
     return rc == 1
 
 

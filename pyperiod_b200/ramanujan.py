@@ -4,8 +4,9 @@
 with the circulant of Ramanujan sums on the FP64 tensor cores (csrc/pp_ramanujan.cu);
 `find_periods_with_weights` thresholds it on the device and hands the selected periods to the
 QOPeriods solve stage (csrc/pp_qo.cu).  fp64 periodograms whose on-chip plan does not fit in shared memory run from
-global memory (csrc/pp_long_ram.cu), with the same folds and the same tensor cores.  Values are fp64; the reference stores its projection in
-float32 (RamanujanPeriods.py:127), so agreement with it is bounded by ~1e-7 relative on the norms.
+global memory (csrc/pp_long_ram.cu), with the same folds and the same tensor cores.  method="divisor" computes the
+same fp64 periodogram from the divisor form of the Ramanujan sums instead (csrc/pp_ram_divisor.cu).  Values are fp64;
+the reference stores its projection in float32 (RamanujanPeriods.py:127), so agreement with it is bounded by ~1e-7 relative on the norms.
 """
 from __future__ import annotations
 
@@ -24,17 +25,28 @@ L2_GROUP_WINDOWS = 1024  # fp64 (fused kernel): windows kept L2-resident while e
 
 
 class RamanujanPeriods(QOPeriods):
-    def __init__(self, basis_type="natural", device=None, precision="fp64", staging="auto"):
+    def __init__(self, basis_type="natural", device=None, precision="fp64", staging="auto", method="dense"):
         """precision (not part of the reference API): "fp64" (FP64 tensor cores, default: the fp64 value of the
         reference's formula), "tf32" (split TF32 contraction on the tcgen05 tensor cores, fp32 accumulation: norms to
         ~1e-5 relative), or "f32_compat" (the reference's own float32 storage and summation order,
         RamanujanPeriods.py:127 and :77-78, reproduced operation by operation: norms equal the reference's to the
         last float32 bit).  staging: see QOPeriods; it applies to the solve stage of find_periods_with_weights.  The
         fp64 periodogram runs on chip when its plan fits in shared memory and from global memory otherwise (the other
-        precisions run on chip only and raise PPError above their limits)."""
+        precisions run on chip only and raise PPError above their limits).
+        method (not part of the reference API): "dense" (default: the circulant contraction above) or "divisor" (the
+        same fp64 norms from the divisor form of the Ramanujan sums, csrc/pp_ram_divisor.cu: a fold and a few comb
+        sums per period instead of a dense product, O(N + q omega(q)) per period instead of O(q^2); values differ from
+        the dense path's by rounding only).  "divisor" needs precision="fp64"; it runs on chip when its plan fits in
+        shared memory and from global memory otherwise."""
+        if method not in ("dense", "divisor"):
+            raise ValueError("method must be 'dense' or 'divisor'")
+        if method == "divisor" and precision != "fp64":
+            raise ValueError("method='divisor' computes the fp64 periodogram only (precision='fp64'): tf32 and "
+                             "f32_compat reproduce the rounding of a dense contraction")
         super().__init__(basis_type, False, False, device=device, staging=staging)
         if precision not in ("fp64", "tf32", "f32_compat"):
             raise ValueError("precision must be 'fp64', 'tf32' or 'f32_compat'")
+        self._method = method
         self._precision = precision
         self._verbose = None
         self._k = 0
@@ -42,9 +54,11 @@ class RamanujanPeriods(QOPeriods):
     # ------------------------------------------------------------------ periodogram
     def _norms_device(self, w, min_length, max_length, _long=None):
         """Norms [B, max_length + 1] on the device.  _long (tests): True forces the global-memory fp64 periodogram,
-        None lets the plan decide."""
+        False the on-chip one, None lets the plan decide."""
         lib = _lib.load()
         tb = get_tables(max_length)
+        if self._method == "divisor":
+            return self._norms_divisor(lib, tb, w, min_length, max_length, _long)
         mu, phi = tb.mu_device(w.device), tb.phi_device(w.device)
         mode = {"fp64": _lib.RAM_FP64, "tf32": _lib.RAM_TF32, "f32_compat": _lib.RAM_F32COMPAT}[self._precision]
         if mode == _lib.RAM_FP64 and _long is None and 1 <= min_length <= max_length <= w.n:
@@ -67,6 +81,22 @@ class RamanujanPeriods(QOPeriods):
               "f32_compat": lib.pp_ramanujan_norms_f32compat}[self._precision]
         call(fn, "pp_ramanujan_norms", w.device, ptr(w.tensor), w.ldx, w.b, w.n, int(min_length), int(max_length),
              ptr(mu), ptr(phi), tb.pmax, tile, ptr(norms), max_length + 1, ptr(ws), ws.numel(), stream_ptr(w.device))
+        return norms
+
+    def _norms_divisor(self, lib, tb, w, min_length, max_length, _long):
+        """The divisor-form periodogram (pp_ramanujan_norms_divisor): shared-memory staging when its plan fits."""
+        spf, phi = tb.spf_device(w.device), tb.phi_device(w.device)
+        staging = _lib.STAGING_AUTO
+        if _long is not None:
+            staging = _lib.STAGING_GLOBAL if _long else _lib.STAGING_SHARED
+        elif 1 <= min_length <= max_length <= w.n:
+            fits = _lib.ramanujan_divisor_fits_on_chip(w.n, min_length, max_length, smem_optin(w.device))
+            staging = _lib.STAGING_SHARED if fits else _lib.STAGING_GLOBAL
+        ws = workspace_for(w.device, lib.pp_ramanujan_divisor_workspace_bytes, w.b, w.n, min_length, max_length)
+        norms = torch.zeros((w.b, max_length + 1), dtype=torch.float64, device=w.device)
+        call(lib.pp_ramanujan_norms_divisor, "pp_ramanujan_norms_divisor", w.device, ptr(w.tensor), w.ldx, w.b, w.n,
+             int(min_length), int(max_length), ptr(spf), ptr(phi), tb.pmax, staging, ptr(norms), max_length + 1,
+             ptr(ws), ws.numel(), stream_ptr(w.device))
         return norms
 
     def find_periods(self, x, min_length=2, max_length=None, select_periods=None):

@@ -72,6 +72,20 @@ def moebius_table(nmax: int) -> np.ndarray:
     return mu
 
 
+def smallest_prime_factor_table(nmax: int) -> np.ndarray:
+    """spf[0..nmax] (spf[0] = 0, spf[1] = 1): the distinct primes of q follow in O(log q) steps (q /= spf[q])."""
+    spf = np.zeros(nmax + 1, dtype=np.int32)
+    if nmax >= 1:
+        spf[1] = 1
+    for p in range(2, int(nmax ** 0.5) + 1):
+        if spf[p] == 0:
+            blk = spf[p * p:: p]
+            blk[blk == 0] = p
+    rest = np.flatnonzero(spf == 0)
+    spf[rest[rest >= 2]] = rest[rest >= 2]
+    return spf
+
+
 def _nontrivial_factor_lists(pmax: int) -> list:
     """nontrivial_factors(n) for every n in 0..pmax, by a sieve.  Each n receives the same insertion sequence as
     _divisor_set builds (every divisor i <= sqrt(n) in ascending order, immediately followed by n // i), so set()
@@ -114,6 +128,7 @@ class PeriodTables:
         self.fac = np.asarray(fac if fac else [0], dtype=np.int32)
         self.phi = euler_phi_table(self.pmax)
         self.mu = moebius_table(self.pmax)
+        self.spf = smallest_prime_factor_table(self.pmax)
         self._dev = {}
         self._dev_phi = {}
 
@@ -137,6 +152,14 @@ class PeriodTables:
         key = "mu:" + str(device)
         if key not in self._dev_phi:
             self._dev_phi[key] = torch.from_numpy(self.mu).to(device)
+        return self._dev_phi[key]
+
+    def spf_device(self, device):
+        """Smallest-prime-factor table as a torch int32 tensor on `device` (cached)."""
+        import torch
+        key = "spf:" + str(device)
+        if key not in self._dev_phi:
+            self._dev_phi[key] = torch.from_numpy(self.spf).to(device)
         return self._dev_phi[key]
 
     def device(self, device):
