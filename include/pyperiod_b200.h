@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PP_ABI_VERSION 10
+#define PP_ABI_VERSION 11
 
 /* sweep metrics */
 #define PP_METRIC_NORM 0   /* ||proj_p|| / sqrt(N)                 Periods.py:221-241, 507-508 */
@@ -434,26 +434,15 @@ int pp_ramanujan_norms_f32compat(const double *x, int64_t ldx, int32_t B, int32_
                                  double *norms, int32_t ld_norms, void *workspace, size_t workspace_bytes,
                                  void *stream);
 
-/* ---- the Ramanujan periodogram of windows that do not fit in shared memory (the "long" path, pp_long_ram.cu) ----
- * pp_ramanujan_fits_on_chip answers, without touching a device, whether the on-chip launch of `mode` (PP_RAM_*) fits
+/* pp_ramanujan_fits_on_chip answers, without touching a device, whether the on-chip launch of `mode` (PP_RAM_*) fits
  * smem_bytes of shared memory per block.  It evaluates the plan the launch itself uses: the fused kernel for
  * PP_RAM_FP64; the fold, contraction and tcgen05 / compat kernels, and N <= 32768 for PP_RAM_F32COMPAT, for the
- * others.  1 = fits, 0 = does not, -1 = bad arguments.
- * pp_long_ramanujan_norms is pp_ramanujan_norms (PP_RAM_FP64) for any N: the same norms from the same folds
- * (summed in increasing n) on the same FP64 tensor cores, with the folds and the Ramanujan sums of a chunk of periods
- * kept in the workspace instead of shared memory.  Batches run in pieces of up to 64 windows and chunks of periods
- * whose folds fit the smaller of half the L2 cache and what the workspace holds (pp_long_ramanujan_workspace_bytes
- * sizes it for 64 MB of folds and Ramanujan sums; it must hold those of period qmax); per-unit partial norms are added in a fixed
- * order, so two runs are bit-identical.  Only columns qmin..qmax of norms[B, ld_norms] are written; nothing is
- * allocated.  The dense work is 2 sum q^2 flop per window: full-range periodograms of N = 2^20 run, slowly. */
+ * others.  1 = fits, 0 = does not, -1 = bad arguments.  An fp64 periodogram that does not fit can be computed by
+ * pp_ramanujan_norms_divisor, for any N. */
 int pp_ramanujan_fits_on_chip(int32_t mode, int32_t N, int32_t qmin, int32_t qmax, int32_t smem_bytes);
-size_t pp_long_ramanujan_workspace_bytes(int32_t B, int32_t N, int32_t qmin, int32_t qmax);
-int pp_long_ramanujan_norms(const double *x, int64_t ldx, int32_t B, int32_t N, int32_t qmin, int32_t qmax,
-                            const int32_t *mu, const int32_t *phi, int32_t table_qmax, double *norms, int32_t ld_norms,
-                            void *workspace, size_t workspace_bytes, void *stream);
 
 /* ---- the Ramanujan periodogram in divisor form (pp_ram_divisor.cu) ---------------------------------------------
- * The same fp64 quantity as pp_ramanujan_norms / pp_long_ramanujan_norms, computed without the dense contraction:
+ * The same fp64 quantity as pp_ramanujan_norms (PP_RAM_FP64), computed without the dense contraction:
  * c_q(n) = sum_{d | gcd(n, q)} mu(q/d) d turns H S_q into an in-place product over the distinct primes p of q,
  *     z = (q / rad(q)) prod_p (p I - A_p) S_q,     (A_p v)_m = sum_{k < p} v[(m + k q / p) mod q],
  * and norms[b, q] = (q / phi(q)^2)^2 sum_m cnt_q[m] z_m^2.  Work per (window, period): the fold (N adds, summed in

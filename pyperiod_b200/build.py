@@ -17,8 +17,8 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_NAME = "libpyperiod_b200.so"
 LIB_PATH = os.path.join(HERE, LIB_NAME)
 SOURCES = ["pp_periods.cu", "pp_qo.cu", "pp_ramanujan.cu", "pp_extract.cu", "pp_bfreq.cu", "pp_comm.cu", "pp_muresan.cu", "pp_microbench.cu", "pp_long.cu",
-           "pp_long_qo.cu", "pp_long_ram.cu", "pp_ram_divisor.cu"]
-HEADERS = ["pp_common.cuh", "pp_sweep.cuh", "pp_host.cuh", "pp_chol.cuh", "pp_cg.cuh", "pp_qo.cuh", "pp_long.cuh", "pp_ram.cuh"]
+           "pp_long_qo.cu", "pp_ram_divisor.cu"]
+HEADERS = ["pp_common.cuh", "pp_sweep.cuh", "pp_host.cuh", "pp_chol.cuh", "pp_cg.cuh", "pp_qo.cuh", "pp_long.cuh"]
 PUBLIC_HEADER = os.path.join(os.path.dirname(HERE), "include", "pyperiod_b200.h")
 
 NVCC_FLAGS = [

@@ -1,5 +1,6 @@
 // pyperiod_b200 -- the fp64 Ramanujan periodogram in divisor form: O(N + q omega(q)) per (window, period) instead of
-// the O(q^2) dense contraction of pp_ramanujan.cu / pp_long_ram.cu.  Same quantity; see DESIGN.md 5.10.
+// the O(q^2) dense contraction of pp_ramanujan.cu, and the fp64 periodogram of every window whose fused on-chip plan
+// does not fit.  Same quantity; see DESIGN.md 5.9 and 5.10.
 //
 //   c_q(n) = sum_{d | gcd(n, q)} mu(q / d) d   =>   (H S_q)_m = sum_{d | q} mu(q / d) d S_d[m mod d]
 //

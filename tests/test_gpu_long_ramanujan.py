@@ -1,8 +1,9 @@
-"""GPU tests of the global-memory ("long") fp64 Ramanujan periodogram (csrc/pp_long_ram.cu).
+"""GPU tests of the default (dense) fp64 Ramanujan periodogram of windows whose fused on-chip plan does not fit: those
+run in divisor form from global memory (csrc/pp_ram_divisor.cu).
 
-(1) the long path forced on windows that fit on chip, against the fp64 closed form and the on-chip path; (2) the
-dispatch at the limit of the on-chip plan; (3)-(5) windows above that limit against the divisor form of the
-periodogram; (6) run-to-run and edge cases; (7) the other precisions keep their limits.
+(1) the divisor form forced on windows that fit on chip, against the fp64 closed form and the fused kernel; (2) the
+dispatch at the limit of the on-chip plan; (3)-(5) windows above that limit against the divisor-form oracle; (6)
+run-to-run and edge cases; (7) the other precisions keep their limits.
 """
 import numpy as np
 import pytest
@@ -39,7 +40,7 @@ def _close(got, want, lo, what):
     assert not bad.any(), (what, np.argwhere(bad)[:5], float((err / np.abs(want[..., lo:])).max()))
 
 
-# ---------------------------------------------------------------- (1) forced long path on windows that fit
+# ---------------------------------------------------------------- (1) forced divisor form on windows that fit
 def test_forced_long_matches_closed_form_and_on_chip():
     n, lo, hi = 999, 3, 333
     xb = synth.synth_batch(70, n, 11)
@@ -74,17 +75,18 @@ def _spy(monkeypatch):
     from pyperiod_b200 import _lib
     lib = _lib.load()
     calls = []
-    for name in ("pp_ramanujan_norms", "pp_long_ramanujan_norms"):
+    for name in ("pp_ramanujan_norms", "pp_ramanujan_norms_divisor"):
         fn = getattr(lib, name)
 
         def spy(*args, _fn=fn, _name=name):
-            calls.append(_name)
+            calls.append(_name if _name == "pp_ramanujan_norms" else (_name, int(args[9])))   # the divisor's staging
             return _fn(*args)
         monkeypatch.setattr(lib, name, spy)
     return calls
 
 
-def test_dispatch_at_the_limit(monkeypatch):
+def test_dispatch_at_the_limit_to_divisor_form(monkeypatch):
+    from pyperiod_b200 import _lib
     n = 9600
     x = synth.synth(n, 21)
     direct = _norms(x, 2, 3200, False)[0]
@@ -94,7 +96,7 @@ def test_dispatch_at_the_limit(monkeypatch):
     assert np.array_equal(at, direct)
     calls.clear()
     above = R().find_periods(x, 2, 3201)
-    assert calls == ["pp_long_ramanujan_norms"]
+    assert calls == [("pp_ramanujan_norms_divisor", _lib.STAGING_GLOBAL)]
     _close(above, norms_divisor_form_f64(x, 2, 3201), 2, "max_length 3201")
 
 

@@ -1,5 +1,5 @@
-"""CPU-only checks of the global-memory Ramanujan periodogram: the divisor-form oracle the long-window GPU tests use,
-the fit query that decides the dispatch (pp_ramanujan_fits_on_chip) and argument errors of pp_long_ramanujan_norms."""
+"""CPU-only checks of the Ramanujan periodogram of long windows: the divisor-form oracle the long-window GPU tests use
+and the fit query that decides the dispatch (pp_ramanujan_fits_on_chip)."""
 import numpy as np
 import pytest
 
@@ -65,33 +65,3 @@ def test_fit_query_rejects_bad_arguments(lib):
     with pytest.raises(_lib.PPError):
         _lib.ramanujan_fits_on_chip(0, 4096, 2, 5000, S)
 
-
-def test_long_argument_errors_do_not_need_a_gpu(lib):
-    d = 16   # a non-null "device pointer": the checks below fail before anything is dereferenced
-    ws = lib.pp_long_ramanujan_workspace_bytes(1, 4096, 2, 1365)
-    assert ws > 0
-    rc = lib.pp_long_ramanujan_norms(d, 4096, 1, 4096, 2, 4097, d, d, 5000, d, 5000, d, ws, None)
-    assert rc == -1 and b"qmax <= N" in lib.pp_last_error()
-    rc = lib.pp_long_ramanujan_norms(d, 4096, 1, 4096, 0, 100, d, d, 5000, d, 5000, d, ws, None)
-    assert rc == -1 and b"qmin" in lib.pp_last_error()
-    rc = lib.pp_long_ramanujan_norms(d, 4096, 1, 4096, 2, 1365, None, d, 1365, d, 1366, d, ws, None)
-    assert rc == -1 and b"tables" in lib.pp_last_error()
-    rc = lib.pp_long_ramanujan_norms(d, 4096, 1, 4096, 2, 1365, d, d, 1000, d, 1366, d, ws, None)
-    assert rc == -1 and b"tables" in lib.pp_last_error()
-    rc = lib.pp_long_ramanujan_norms(d, 4096, 1, 4096, 2, 1365, d, d, 1365, d, 1365, d, ws, None)
-    assert rc == -1 and b"leading dimension" in lib.pp_last_error()
-    rc = lib.pp_long_ramanujan_norms(None, 4096, 1, 4096, 2, 1365, d, d, 1365, d, 1366, d, ws, None)
-    assert rc == -1
-    rc = lib.pp_long_ramanujan_norms(d, 0, 1, 4096, 2, 1365, d, d, 1365, d, 1366, d, ws, None)
-    assert rc == -1
-    rc = lib.pp_long_ramanujan_norms(d, 4096, 1, 4096, 2, 1365, d, d, 1365, d, 1366, d, 4096, None)
-    assert rc == -3 and b"workspace" in lib.pp_last_error()
-    rc = lib.pp_long_ramanujan_norms(d, 4096, 1, 4096, 2, 1365, d, d, 1365, d, 1366, None, ws, None)
-    assert rc == -3
-    # empty batches are accepted without looking at anything else
-    assert lib.pp_long_ramanujan_norms(None, 0, 0, 0, 0, 0, None, None, 0, None, 0, None, 0, None) == 0
-    assert lib.pp_long_ramanujan_workspace_bytes(1, 4096, 2, 4097) == 0
-    assert lib.pp_long_ramanujan_workspace_bytes(1, 4096, 0, 100) == 0
-    # the workspace does not grow with qmax^2: 64 MB of folds and Ramanujan sums (plus partial norms) at any N
-    assert lib.pp_long_ramanujan_workspace_bytes(1, 1 << 20, 2, (1 << 20) // 3) < (80 << 20)
-    assert lib.pp_long_ramanujan_workspace_bytes(64, 131072, 2, 43690) < (80 << 20)
