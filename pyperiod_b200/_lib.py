@@ -151,26 +151,37 @@ FOLD_NAMES = {"hierarchical": FOLD_HIERARCHICAL, "direct": FOLD_DIRECT, "no_ride
 # The C library keeps no process-wide state: the fold mode and the optional profile buffer are arguments of every
 # call.  These two module variables are only the DEFAULTS the Python classes pass when an instance does not set
 # its own (`Periods(..., fold_mode=...)`); tests and the tuning tools use them to switch whole scripts.
-_default_fold_mode = FOLD_HIERARCHICAL
+# None = no fold mode named: the hierarchy, except that plain M-best then ranks with the fp32 nomination
+# (Periods._fold).  A mode named with set_fold_mode, FOLD_HIERARCHICAL included, applies to every call.
+_module_fold_mode = None
 _profile_ptr = 0
 
 
-def set_fold_mode(mode: int):
-    """Default fold mode of instances that do not choose one (FOLD_*; see include/pyperiod_b200.h)."""
-    global _default_fold_mode
+def set_fold_mode(mode):
+    """Default fold mode of instances that do not choose one (FOLD_*; see include/pyperiod_b200.h).  None returns to
+    the unset default."""
+    global _module_fold_mode
+    if mode is None:
+        _module_fold_mode = None
+        return
     if int(mode) not in FOLD_NAMES.values():
         raise PPError("unknown fold mode")
-    _default_fold_mode = int(mode)
+    _module_fold_mode = int(mode)
+
+
+def fold_mode_is_set() -> bool:
+    """Whether set_fold_mode named a module-wide fold mode."""
+    return _module_fold_mode is not None
 
 
 def default_fold_mode() -> int:
-    return _default_fold_mode
+    return FOLD_HIERARCHICAL if _module_fold_mode is None else _module_fold_mode
 
 
 def resolve_fold_mode(mode) -> int:
     """None -> the module default; a FOLD_* value or one of FOLD_NAMES."""
     if mode is None:
-        return _default_fold_mode
+        return default_fold_mode()
     if isinstance(mode, str):
         return FOLD_NAMES[mode]
     return int(mode)

@@ -69,7 +69,12 @@ struct SmemPlan {
   __host__ __device__ size_t bytes() const { return off_nom() + (tie_len ? (size_t)skip_words * 4 : 0) + 16; }
 };
 
-constexpr int kF32Pad = 320;  // floats after the window in the fp32 copies: masked 64-wide tiles read past N
+// Floats after the window in the fp32 copies, all zero.  A masked tile of JR pair columns starting at ra < g reads
+// the elements up to ra + 64 JR - 1 of each complete row, i.e. up to N + 64 JR - 2 in row M0 - 1 (the tail row only
+// reads pairs that start below N).  The widest masked tile is half a top tile at L = 0: 4 pair columns, 256 floats.
+constexpr int kF32Pad = 320;
+static_assert(kF32Pad >= 64 * (hier_cols_f32<0>::value / 2) && kF32Pad >= 64,
+              "the masked fp32 tiles must not read past the zero tail of the float copies");
 
 __host__ __device__ inline SmemPlan make_plan(int N, int pmax, int num, bool sweep_pad, bool hier = false,
                                               bool f32 = false, bool tie = false) {
@@ -133,6 +138,9 @@ __device__ __forceinline__ void refresh_f32_copies(const double* xs, int N, floa
     if (n > 0) xf1[n - 1] = v;
   }
 }
+
+// e >= the sum of squares that cta_sum_sq rounded to `s` (N fma terms: relative error below N 2^-53)
+__device__ __forceinline__ double f32_sum_sq_bound(double s, int N) { return fma(s, (double)(N + 2) * 0x1p-52, s); }
 
 __device__ __forceinline__ void zero_pad(double* xs, int from, int to) {
   for (int i = from + threadIdx.x; i < to; i += kThreads) xs[i] = 0.0;
@@ -312,7 +320,7 @@ mbest_kernel(const double* __restrict__ x, int64_t ldx, int B, int N, int num, i
              int trunc_i, int orth_i, int hier, Tables tb, uint32_t* __restrict__ periods_out, double* __restrict__ powers_out,
              double* __restrict__ bases_out, int32_t* __restrict__ sweeps_out, int32_t* __restrict__ status_out,
              double* __restrict__ ws_slots, double* __restrict__ ws_scr, const uint2* __restrict__ tops, int ntops,
-             int* __restrict__ next_window, unsigned long long* __restrict__ prof, int f32, double* __restrict__ ws_keys,
+             int* __restrict__ next_window, unsigned long long* __restrict__ prof, int f32,
              int32_t* __restrict__ near_ties_out) {
   unsigned char* smem_raw = pp_smem;
   const SmemPlan pl = make_plan(N, pmax, num, true, hier != 0, f32 != 0, true);
@@ -345,7 +353,10 @@ mbest_kernel(const double* __restrict__ x, int64_t ldx, int B, int N, int num, i
     loader.load(sm.xs, x + (size_t)b * ldx, N);
     const double e_data = cta_sum_sq(sm.xs, N, sm.red);
     const double data_norm = sqrt(e_data) / sqrtN;  // periodic_norm(data), Periods.py:600
-    if (sm.xf0 != nullptr) refresh_f32_copies(sm.xs, N, sm.xf0, sm.xf1);  // published by the barrier below
+    // fp32 nomination only while no float value of a sweep can overflow: every residue sum and tile energy stays
+    // below N sum x^2 (f32_energy_tol); other windows (and NaN / Inf data) rank with the fp64 hierarchy
+    const bool f32_win = F32 && sm.xf0 != nullptr && (double)N * e_data <= 0x1p120;
+    if (f32_win) refresh_f32_copies(sm.xs, N, sm.xf0, sm.xf1);  // published by the barrier below
     if (threadIdx.x == 0) {
       misc[0] = 0;
       misc[1] = 0;
@@ -372,9 +383,9 @@ mbest_kernel(const double* __restrict__ x, int64_t ldx, int B, int N, int num, i
       sp.warp_scr = my_scr;
       sp.pv = pl.pv;
       sp.sqrtN = sqrtN;
-      // fp32 nomination: the residual of an orthogonal projection never has more energy than the data, so the
-      // data's energy bounds the float error of every sweep of this window
+      // bound of the near-tie audit: the residual of an orthogonal projection never has more energy than the data
       sp.e_res = e_data;
+      sp.e_f32 = f32_sum_sq_bound(e_data, N);
       sp.data_norm = 1.0;
       sp.thresh = -1.0;
       sp.skip = sm.skip;
@@ -385,9 +396,11 @@ mbest_kernel(const double* __restrict__ x, int64_t ldx, int B, int N, int num, i
       sp.rcp = sm.sweep->rcp;
       sp.tops = tops;
       sp.ntops = ntops;
-      sp.verify_keys = sm.xf0 != nullptr ? ws_keys + (size_t)blockIdx.x * (pmax + 2) : nullptr;
-      sp.xf0_off = sm.xf0 != nullptr ? (int)pl.off_xf() : 0;
-      sp.xf1_off = sm.xf0 != nullptr ? (int)(pl.off_xf() + (size_t)pl.xf_len * 4) : 0;
+      // the float keys share the near-tie audit's key array: cta_sweep is done with them before the audit's keys
+      // are written
+      sp.verify_keys = f32_win ? sm.tie_keys : nullptr;
+      sp.xf0_off = f32_win ? (int)pl.off_xf() : 0;
+      sp.xf1_off = f32_win ? (int)(pl.off_xf() + (size_t)pl.xf_len * 4) : 0;
       sp.tie_keys = sm.tie_keys;
       sp.tie_nom = sm.tie_nom;
       sp.canon_v = sm.vwin;
@@ -458,9 +471,12 @@ mbest_kernel(const double* __restrict__ x, int64_t ldx, int B, int N, int num, i
         }
       }
       cta_subtract_tiled(sm.xs, N, sm.vwin, top.p);  // always (:537)
-      if (sm.xf0 != nullptr) {
+      if (f32_win) {
         __syncthreads();
         refresh_f32_copies(sm.xs, N, sm.xf0, sm.xf1);
+        // the next sweep's float error scales with the residual's energy, which falls round by round
+        const double e_now = cta_sum_sq(sm.xs, N, sm.red);
+        if (threadIdx.x == 0) sm.sweep->params.e_f32 = f32_sum_sq_bound(e_now, N);
       }
       __syncthreads();
       { const long long t = clock64(); t_upd += t - t_mark; t_mark = t; }
@@ -920,7 +936,7 @@ size_t pp_workspace_bytes(int32_t algo, int32_t N, int32_t pmax, int32_t num, in
   // upper bound on the persistent grid
   const size_t grid = (size_t)f.sm_count * (algo == PP_ALGO_S2L ? kS2lCtasPerSm : kCtasPerSm);
   size_t bytes = 1024 + 1024 + (size_t)(pmax + 2) * sizeof(uint2);
-  if (algo == PP_ALGO_MBEST) bytes += grid * ((size_t)num * pl.pv + (size_t)(pmax + 2)) * 8;
+  if (algo == PP_ALGO_MBEST) bytes += grid * (size_t)num * pl.pv * 8;
   if (orth && algo != PP_ALGO_BCORR) bytes += grid * kWarps * 2 * (size_t)pl.pv * 8;
   if (algo == PP_ALGO_BCORR) bytes += grid * (size_t)(pmax + 2) * 8;  // hierarchical keys awaiting verification
   return bytes;
@@ -1059,8 +1075,6 @@ int pp_mbest(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t num, in
   if (int rc = prep_kernel(kernel, pl.bytes(), f)) return rc;
   const int grid = grid_for(f, pl.bytes(), B);
   size_t off = 0;
-  double* keys = f32 ? carve(workspace, workspace_bytes, off, (size_t)grid * (pmax + 2) * 8) : nullptr;
-  if (f32 && !keys) return fail(-3, "workspace too small (see pp_workspace_bytes)%s");
   double* slots = carve(workspace, workspace_bytes, off, (size_t)grid * num * pl.pv * 8);
   double* scr = orth ? carve(workspace, workspace_bytes, off, (size_t)grid * kWarps * 2 * pl.pv * 8) : nullptr;
   if (!slots || (orth && !scr)) return fail(-3, "workspace too small (see pp_workspace_bytes)%s");
@@ -1078,7 +1092,7 @@ int pp_mbest(const double* x, int64_t ldx, int32_t B, int32_t N, int32_t num, in
   kernel<<<grid, kThreads, pl.bytes(), (cudaStream_t)stream>>>(x, ldx, B, N, num, pmin, pmax, gamma, trunc, orth,
                                                                      hier, tb, periods, powers, bases, sweeps, status,
                                                                      slots, scr, tops, ntops, next_window,
-                                                                     reinterpret_cast<unsigned long long*>(profile), f32, keys,
+                                                                     reinterpret_cast<unsigned long long*>(profile), f32,
                                                                      near_ties);
   return check_cuda(cudaGetLastError(), "mbest_kernel launch");
 }

@@ -52,6 +52,7 @@ struct SweepParams {
   double sqrtN;
   double e_res;       // ||residual||^2   (IMPOSED)
   double data_norm;   // ||x||/sqrt(N)    (IMPOSED)
+  double e_f32;       // >= sum x^2 of the swept signal: scale of the fp32 nomination's error bound (f32_energy_tol)
   double thresh;      // IMPOSED early-stop threshold; <0 disables first-hit mode
   const uint32_t* skip;  // bitmap of periods to ignore (M-best), nullable
   int nskip;             // number of bits set in skip (0 => the bitmap is not consulted)
@@ -61,10 +62,10 @@ struct SweepParams {
   const double* rcp;     // shared table rcp[m] = 1.0 / m for m < kRcpTab (energy weights without a division)
   const uint2* tops;     // global: descriptors of the hierarchical tops in hand-out order (tops_kernel)
   int ntops;
-  double* verify_keys;   // global [pmax+1], nullable: lets MAXABS sweeps rank hierarchically (needs e_res = sum x^2)
+  double* verify_keys;   // [pmax+1] (global or shared), nullable: lets MAXABS sweeps rank hierarchically (needs e_res = sum x^2)
   // fp32 nomination (NORM / GAMMA ranking sweeps): two float copies of the window in shared memory, xf1[n] = x[n+1],
   // so that a pair of consecutive samples can always be read with one aligned 8-byte load.  Needs verify_keys
-  // and e_res >= sum x^2.  offset 0 => fp64 hierarchical sweep.
+  // and e_f32 >= sum x^2 of the swept signal.  offset 0 => fp64 hierarchical sweep.
   // (byte offsets into the kernel's dynamic shared memory, so that the loads stay LDS; 0 = none)
   int xf0_off;
   int xf1_off;
@@ -823,17 +824,16 @@ __device__ __forceinline__ void warp_hier_rider_L(RankCtx rc, int g, int M0, int
 // fp32 nomination sweep
 // ------------------------------------------------------------------------------------------
 // The same jobs (tops, chains, riders) evaluated in float: a lane owns the residue PAIR ra + 2 lane + 64 j + {0, 1},
-// one aligned LDS.64 feeds two FADDs, so a pass costs half the shared-memory wavefronts and half the
+// one aligned LDS.64 feeds one FADD2, so a pass costs half the shared-memory wavefronts and half the
 // instructions of the fp64 pass.  The float energies only NOMINATE: cta_sweep re-evaluates every candidate whose
 // upper bound reaches the best lower bound with the sequential fp64 fold, so the selected period and its norm are
 // those of the exact fold (pp_sweep.cuh: cta_sweep).
 struct F32Window {
   int off0;  // byte offset in pp_smem of x0[n] = (float) x[n]
   int off1;  // byte offset in pp_smem of x1[n] = (float) x[n + 1]
-  // aligned pointer to the pairs (e + 2 lane, e + 2 lane + 1), e = element index of the pair owned by lane 0
-  __device__ __forceinline__ const float2* row(int e) const {
-    const int byte = (e & 1) ? off1 + 4 * (e - 1) : off0 + 4 * e;
-    return reinterpret_cast<const float2*>(pp_smem + byte) + (threadIdx.x & 31);
+  // byte offset of the aligned pair (e + 2 lane, e + 2 lane + 1), e = element index of the pair owned by lane 0
+  __device__ __forceinline__ int pair_byte(int e) const {
+    return ((e & 1) ? off1 + 4 * (e - 1) : off0 + 4 * e) + 8 * (threadIdx.x & 31);
   }
 };
 
@@ -929,38 +929,76 @@ struct rider_levels_f32 {
 };
 
 // rows (stride g) of the base-residue pairs ra + 2 lane + 64 j + {0, 1} into S sets by (row - M0) mod S, plus the
-// predicated tail row into set 0; lanes / components past g are zeroed when MASK.
+// tail row into set 0; lanes / components past g are zeroed when MASK.  As in hier_accumulate, the first complete
+// group of S rows initialises the sets (no zero fill) and the `head` rows before it come last.
+// Row k starts at element ra + k g: its pair sits at (k odd ? po : pe) + 4 k g bytes.  For even g both are the same
+// copy of the window; for odd g the rows alternate between the two copies.  So rows of one parity are one pointer
+// that advances 8 g bytes per row, and every row costs one LDS.64 per column plus one address add.
+template <int J>
+__device__ __forceinline__ void load_row_f32(float2 (&acc)[J], const unsigned char* row) {
+  const float2* r = reinterpret_cast<const float2*>(row);
+#pragma unroll
+  for (int j = 0; j < J; ++j) acc[j] = r[32 * j];
+}
 template <int S, int J, bool MASK>
 __device__ __forceinline__ void hier_accumulate_f32(const F32Window& w, int g, int ra, int M0, int rr, int head,
                                                     int groups, float2 (&acc)[S][J], bool (&tail)[J][2]) {
   const int lane = threadIdx.x & 31;
-#pragma unroll
-  for (int s = 0; s < S; ++s)
-#pragma unroll
-    for (int j = 0; j < J; ++j) acc[s][j] = make_float2(0.f, 0.f);
-  int e = ra;
+  const int g4 = 4 * g, g8 = 8 * g;
+  const unsigned char* pe = pp_smem + w.pair_byte(ra);
+  const unsigned char* po = pp_smem + w.pair_byte(ra + g) - g4;
+  const unsigned char* tail_row;
   if constexpr (S == 1) {
-#pragma unroll 2
-    for (int k = 0; k < M0; ++k) {
-      add_row_f32<J>(acc[0], w.row(e));
-      e += g;
+    load_row_f32<J>(acc[0], pe);
+    const unsigned char* qo = po + g4;  // row 1
+    const unsigned char* qe = pe + g8;  // row 2
+#pragma unroll 1
+    for (int k = (M0 - 1) >> 1; k > 0; --k) {
+      add_row_f32<J>(acc[0], reinterpret_cast<const float2*>(qo));
+      add_row_f32<J>(acc[0], reinterpret_cast<const float2*>(qe));
+      qo += g8;
+      qe += g8;
     }
-  } else {
+    if (!(M0 & 1)) add_row_f32<J>(acc[0], reinterpret_cast<const float2*>(qo));  // row M0 - 1
+    tail_row = (M0 & 1) ? qo : qe;
+  } else {  // S is even
+    const unsigned char* qe = ((head & 1) ? po : pe) + head * g4;  // rows head + even s
+    const unsigned char* qo = ((head & 1) ? pe : po) + (head + 1) * g4;  // rows head + odd s
 #pragma unroll
-    for (int s = 1; s < S; ++s) {  // rows before the first complete group of S
-      if (s >= S - head) {
-        add_row_f32<J>(acc[s], w.row(e));
-        e += g;
+    for (int s = 0; s < S; ++s) {
+      if (s & 1) {
+        load_row_f32<J>(acc[s], qo);
+        qo += g8;
+      } else {
+        load_row_f32<J>(acc[s], qe);
+        qe += g8;
       }
     }
 #pragma unroll 1
-    for (int i = groups; i > 0; --i) {
+    for (int i = groups - 1; i > 0; --i) {
 #pragma unroll
       for (int s = 0; s < S; ++s) {
-        add_row_f32<J>(acc[s], w.row(e));
-        e += g;
+        if (s & 1) {
+          add_row_f32<J>(acc[s], reinterpret_cast<const float2*>(qo));
+          qo += g8;
+        } else {
+          add_row_f32<J>(acc[s], reinterpret_cast<const float2*>(qe));
+          qe += g8;
+        }
       }
     }
+    const unsigned char* hc = pe;       // head rows 0, 1, ... into sets S - head .. S - 1
+    const unsigned char* hn = po + g4;
+#pragma unroll
+    for (int s = 1; s < S; ++s) {
+      if (s >= S - head) {  // warp-uniform
+        add_row_f32<J>(acc[s], reinterpret_cast<const float2*>(hc));
+        const unsigned char* t = hn;
+        hn = hc + g8;
+        hc = t;
+      }
+    }
+    tail_row = qe;  // row head + groups S = M0
   }
 #pragma unroll
   for (int j = 0; j < J; ++j) {
@@ -969,13 +1007,14 @@ __device__ __forceinline__ void hier_accumulate_f32(const F32Window& w, int g, i
     tail[j][1] = r + 1 < rr;
   }
   if (ra < rr) {  // warp-uniform
-    const float2* row = w.row(e);
+    // one predicate per pair: the tail row of a pair starting below rr may reach element N, which is zero in both
+    // copies; the pair of a residue >= rr can lie past the zero pad
+    const float2* row = reinterpret_cast<const float2*>(tail_row);
 #pragma unroll
     for (int j = 0; j < J; ++j) {
       float2 t = make_float2(0.f, 0.f);
-      if (tail[j][0]) t = row[32 * j];  // predicated: the tail row of a residue >= rr lies past the window
-      acc[0][j].x += t.x;
-      acc[0][j].y += tail[j][1] ? t.y : 0.f;
+      if (tail[j][0]) t = row[32 * j];
+      acc[0][j] = add_f32x2(acc[0][j], t);
     }
   }
   if (MASK) {
@@ -1055,14 +1094,14 @@ __device__ __forceinline__ void rider_tile_f32(const F32Window& w, int g, int ra
   fold_partial<LH>(Tr, Ar, t, a);
 }
 
-// columns (of 64 residues) per accumulator set: 8 float accumulators per lane for L <= 2, 16 for L = 3
-#ifndef PP_F32_COLS0
-#define PP_F32_COLS0 4
-#endif
+// columns (of 64 residues) per accumulator set: 16 float accumulators per lane (8 / 4 / 2 / 1 columns for L = 0..3),
+// the register budget of the fp64 tiles, so a float tile covers twice their residues.  What is left of a top after
+// the full tiles runs as masked tiles of half the width (one or two of them).
 template <int L>
 struct hier_cols_f32 {
-  static constexpr int value = (PP_F32_COLS0 >> L) > 1 ? (PP_F32_COLS0 >> L) : 1;
+  static constexpr int value = (8 >> L) > 1 ? (8 >> L) : 1;
 };
+constexpr int kRiderColsF32 = 2;  // rider tiles: 3 * 2^LH sets of 2 columns
 
 // float energies of one top and its chain, written to keys[] (no ranking here)
 template <int L>
@@ -1077,12 +1116,9 @@ __device__ __forceinline__ void warp_hier_top_f32(const RankCtx& rc, const F32Wi
 #pragma unroll
   for (int i = 0; i <= L; ++i) T[i] = A[i] = 0.0;
   int ra = 0;
+  constexpr int JR = J > 1 ? J / 2 : 1;
   for (; ra + 64 * J <= g; ra += 64 * J) hier_tile_f32<L, J, false>(w, g, ra, M0, rr, T, A, out);
-#ifdef PP_F32_REM2
-  if constexpr (J > 2)
-    for (; ra + 128 <= g; ra += 128) hier_tile_f32<L, 2, false>(w, g, ra, M0, rr, T, A, out);
-#endif
-  for (; ra < g; ra += 64) hier_tile_f32<L, 1, true>(w, g, ra, M0, rr, T, A, out);
+  for (; ra < g; ra += 64 * JR) hier_tile_f32<L, JR, true>(w, g, ra, M0, rr, T, A, out);
   constexpr int KP = L == 0 ? 1 : (L == 1 ? 2 : 4);
   double e[KP];
 #pragma unroll
@@ -1151,7 +1187,8 @@ __device__ __forceinline__ void warp_hier_rider_f32(const RankCtx& rc, const F32
 #pragma unroll
   for (int i = 0; i < LH; ++i) Tr[i] = Ar[i] = 0.0;
   int ra = 0;
-  for (; ra + 64 <= g; ra += 64) rider_tile_f32<LH, 1, false>(w, g, ra, M0, rr, head, groups, Th, Ah, Tr, Ar);
+  constexpr int J = kRiderColsF32;
+  for (; ra + 64 * J <= g; ra += 64 * J) rider_tile_f32<LH, J, false>(w, g, ra, M0, rr, head, groups, Th, Ah, Tr, Ar);
   for (; ra < g; ra += 64) rider_tile_f32<LH, 1, true>(w, g, ra, M0, rr, head, groups, Th, Ah, Tr, Ar);
   constexpr int NV = 2 * LH + 1;
   constexpr int KP = NV <= 4 ? 4 : 8;
@@ -1196,12 +1233,28 @@ __device__ __forceinline__ void warp_hier_job_f32(const RankCtx& rc, const F32Wi
   }
 }
 
-// Upper bound of |float energy - exact energy| of candidate p (first-order, doubled): input rounding, the float
-// summation of ceil(N/p) terms per residue (any order), the float squares and per-tile energy sums (<= 40 u);
-// everything relative to sum x^2 because sum_r (sum_{i in r} |x_i|)^2 / cnt_r <= sum x^2 (Cauchy-Schwarz).
-__device__ __forceinline__ double f32_energy_tol(int N, int p, double e_res) {
-  const double u = 5.9604644775390625e-08;  // 2^-24
-  return 2.0 * (2.0 * (double)((N + p - 1) / p) + 40.0) * u * e_res;
+// Upper bound of |float key - exact energy| of candidate p.  c = ceil(N/p), M = floor(N/p), u = 2^-24, e >= sum x^2 of
+// the swept signal, K = kF32TileTerms: the float terms one lane sums per tile and level (2 components x J columns x
+// S sets of that level).
+//   residue sums  S_r adds its c_r <= c samples in float, in any order, after rounding them to float:
+//                 |dS_r| <= c_r u A_r with A_r = sum_{i in r} |x_i|, so |d(S_r^2 / c_r)| <= 2 u A_r^2 <= 2 c u e_r
+//                 (Cauchy-Schwarz: A_r^2 <= c_r e_r, e_r = sum_{i in r} x_i^2), 2 c u e over all residues;
+//   tile sums     a tile's float T and A of one level each sum at most K rounded squares (relative error K u); the
+//                 key T / M + (1/(M+1) - 1/M) A then moves by K u (T / M + A / (M (M+1))) <= K u (M + 2) / M E,
+//                 since T <= (M + 1) E and A <= T, with E <= e the candidate's energy;
+//   underflow     gradual underflow adds at most 2^-150 to each rounded sample and square (float sums round exactly
+//                 below 2^-126): 2^-149 (sum |x| + p) <= 2^-149 (N + e + p).
+// The tile partials are summed and weighted in double, which the doubling of this first-order bound covers.  Every
+// float value stays below c e <= N e, so the caller must keep N e below the float range (mbest_kernel: 2^120).
+constexpr int kF32TileTerms = 24;
+static_assert(2 * 8 <= kF32TileTerms && 2 * (1 << 2) * kRiderColsF32 <= kF32TileTerms &&
+                  2 * (3 << 1) * kRiderColsF32 <= kF32TileTerms,
+              "tops hold 8 pairs per lane and level, riders 2^LH (host) or 3 * 2^(LH-1) (rider) sets of pairs");
+__device__ __forceinline__ double f32_energy_tol(int N, int p, double e) {
+  const double u = 0x1p-24;
+  const int M = N / p, c = (N + p - 1) / p;
+  const double terms = 2.0 * (double)c + (double)kF32TileTerms * (double)(M + 2) / (double)M;
+  return 2.0 * (terms * u * e + 0x1p-149 * ((double)N + (double)p + e));
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1433,7 +1486,7 @@ static __device__ __noinline__ SweepResult cta_sweep(SweepShared* sh) {
     }
     if (threadIdx.x == 0) sh->ncand = 0;
     __syncthreads();  // every float energy is in keys[]
-    const double e_res = sp->e_res;
+    const double e_res = sp->e_f32;
     const bool gam = metric == PP_METRIC_GAMMA;
     const uint32_t* skip = rc.skip;
     double lb = -1.0;  // best guaranteed lower bound of a ranking value

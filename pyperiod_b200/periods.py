@@ -114,8 +114,10 @@ class Periods:
         worker thread and one set of launches per device, results concatenated on the host (windows are independent:
         no collective; the one-process-per-GPU form of the same sharding is pyperiod_b200.sharding).  dtype="fp32" ranks the M-best sweeps in float
         (half the shared-memory traffic) and re-folds every candidate inside the float error bound in fp64, so the
-        period lists and norms are those of the fp64 path (the north star's fp32 option).  fold_mode (a
-        _lib.FOLD_* value or name) picks how ranking sweeps obtain the residue sums; None = the module default.
+        period lists and norms are those of the fp64 path (the north star's fp32 option).  The plain M-best calls
+        (neither trunc nor orth) rank that way with the default dtype too.  fold_mode (a _lib.FOLD_* value or name)
+        picks how ranking sweeps obtain the residue sums; None = the module default (and the fp32 nomination for
+        plain M-best while no module default is set).
 
         staging picks where a window lives while it is processed.  "shared" stages it in one CTA's shared memory (the
         on-chip kernels; a window whose plan does not fit raises PPError).  "global" runs the global-memory path: the
@@ -150,9 +152,14 @@ class Periods:
         self._staging = staging
         _lib.load()  # fail loudly now if the CUDA library is missing
 
-    def _fold(self) -> int:
-        """Fold mode of this instance's calls (per-call argument of the C ABI)."""
-        if self._fold_mode is None and self._dtype == "fp32":
+    def _fold(self, plain_mbest: bool = False) -> int:
+        """Fold mode of this instance's calls (per-call argument of the C ABI).  plain_mbest: an M-best call with
+        neither trunc nor orth.  Unless the instance or the module (_lib.set_fold_mode) names a fold mode, those rank
+        with the fp32 nomination sweep: its float energies only nominate, and every candidate they cannot
+        separate from the best is refolded in fp64, so the periods are those of the fp64 sweeps at half the
+        shared-memory traffic."""
+        if self._fold_mode is None and (self._dtype == "fp32" or
+                                        (plain_mbest and not _lib.fold_mode_is_set())):
             return _lib.FOLD_NOMINATE_F32
         return _lib.resolve_fold_mode(self._fold_mode)
 
@@ -330,9 +337,12 @@ class Periods:
         tb = get_tables(pmax)
         co, cq, fo, fc = tb.device(w.device)
         orth = int(self._orthogonalize)
-        fold = self._fold()
         trunc = int(self._trunc_to_integer_multiple)
         metric = _lib.METRIC_GAMMA if gamma else _lib.METRIC_NORM
+        fold = self._fold(plain_mbest=not trunc and not orth)
+        if fold != self._fold() and not _lib.fits_on_chip(_lib.ALGO_MBEST, w.n, pmax, num, metric, trunc, orth, fold,
+                                                          smem_optin(w.device)):
+            fold = self._fold()   # no room on chip for the float copies of the window: rank with the fp64 hierarchy
         long = _global_staging(self._staging, w.device, _lib.ALGO_MBEST, w.n, pmax, num, metric, trunc, orth, fold)
         if long:
             ws = workspace_for(w.device, lib.pp_long_workspace_bytes, _lib.ALGO_MBEST, w.b, w.n, pmax, num, orth)

@@ -1,4 +1,7 @@
-"""Quick device-resident throughput probe (not the contract bench): python tools/perf_mbest.py [B]"""
+"""Quick device-resident throughput probe (not the contract bench): python tools/perf_mbest.py [B] [modes]
+
+modes: comma-separated, run in the order given (repeat them to alternate): hier, direct, norider, f32, or default
+(Periods() without a fold mode, which ranks plain M-best with the fp32 nomination sweep)."""
 import sys, time, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -10,11 +13,12 @@ stream = synth.synth_stream(B)
 dev = torch.from_numpy(stream).cuda()
 win = torch.as_strided(dev, (B, 4096), (512, 1))
 TRUNC = os.environ.get("PP_TRUNC", "0") == "1"      # PP_TRUNC=1: Periods(True, False), the truncated fold
-P = Periods(True, False) if TRUNC else Periods()
 prof = torch.zeros(8, dtype=torch.int64, device="cuda")
 _lib.set_profile_buffer(prof)
 for mode in modes:
-    _lib.set_fold_mode({"direct": _lib.FOLD_DIRECT, "norider": _lib.FOLD_HIERARCHICAL_NO_RIDERS, "f32": _lib.FOLD_NOMINATE_F32}.get(mode, _lib.FOLD_HIERARCHICAL))
+    fold = {"direct": _lib.FOLD_DIRECT, "norider": _lib.FOLD_HIERARCHICAL_NO_RIDERS, "f32": _lib.FOLD_NOMINATE_F32,
+            "hier": _lib.FOLD_HIERARCHICAL, "default": None}[mode]
+    P = Periods(True, False, fold_mode=fold) if TRUNC else Periods(fold_mode=fold)
     for name, fn in (("m_best", P.m_best), ("m_best_gamma", P.m_best_gamma)):
         fn(win, num=10, max_length=1024)
         fn(win, num=10, max_length=1024)
